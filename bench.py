@@ -9,7 +9,7 @@ getCost(c, new_control=false): forward sweep + backward sweep (400 Trotter steps
 fidelity overlaps and the basis projections.  Controls are synthetic (seeded); psi_init / psi_target are
 the DMRG ground-state fixtures shipped in optimalcontrolmps_b200/data.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--hessian-nt NT]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--hessian-nt NT] [--dump-outputs DIR]
 
 N>1 (torchrun): every rank evaluates its own control on its own GPU (independent units, weak scaling);
 the (cost, gradient) tuples are combined with one NCCL all-gather.  --impl reference times the CPU
@@ -335,6 +335,8 @@ def run_ours(args):
     sampler.stop_flag = True
     if rank == 0:
         sampler.join(timeout=2)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, ocp, list(c), *res)
     # max over ranks of the device-timed region and of the end-to-end wall clock
     tt = torch.tensor([dev_ms * 1e-3, wall], dtype=torch.float64, device=dev)
     if world > 1:
@@ -442,6 +444,23 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_outputs(path, ocp, c, cost, grad):
+    """What the last timed evaluation computed, as float64 arrays `path/<name>.npy` (a few kB in all): the cost and the gradient
+    the caller receives, divT (overlap derivative at every time point, real / imaginary columns), the fidelity of every slice of
+    psi_t and the bond dimensions of every slice of psi_t and xi_t.  The inputs depend on --seed only, so two builds of the
+    project can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    out = {"cost": np.array([cost], dtype=np.float64),
+           "gradient": np.asarray(grad, dtype=np.float64),
+           "divT": np.ascontiguousarray(ocp.divT, dtype=np.complex128).view(np.float64).reshape(-1, 2),
+           "fidelities": np.asarray(ocp.getFidelityForAllT(c, False), dtype=np.float64),   # overlaps of the stored psi_t, no new sweep
+           "psi_bond_dims": np.asarray(ocp.psi_t.bond_dims(), dtype=np.float64),
+           "xi_bond_dims": np.asarray(ocp.xi_t.bond_dims(), dtype=np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log(f"cfg2: outputs of the last timed evaluation written to {path}")
 
 
 def batched_bench(B, oc, st, psi_i, psi_f, ocp0, c0):
@@ -771,7 +790,13 @@ def main():
     ap.add_argument("--cfg5", type=int, default=1, help="1: add the cfg5 block (L=50 chi=256 bounded sample; N=1 only)")
     ap.add_argument("--cfg4-seeds", type=int, default=8, help="controls per GPU of the cfg4 block (L=30 chi=150 batched seeds); 0 = off")
     ap.add_argument("--cfg4-inflight", type=int, default=8, help="cfg4 controls evaluated concurrently per GPU at most (21 GB of slice stores each; limited by the free device memory)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last timed cfg2 evaluation computed "
+                                                          "(rank 0) as DIR/<name>.npy; GPU arm only")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

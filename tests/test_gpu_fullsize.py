@@ -123,6 +123,35 @@ def test_cfg2_full_evaluation_matches_golden(cfg2):
     assert np.array_equal(g.xi_t.bond_dims(), z["xi_dims"])
 
 
+def test_bench_dump_outputs_match_golden(tmp_path):
+    """bench.py --dump-outputs writes what its last timed evaluation computed.  At the default seed that is the evaluation of
+    golden_cfg2_eval.npz: cost and fidelities 1e-9, gradient and divT 1e-7, every bond dimension, and the cost of the JSON line."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from conftest import ROOT, load_golden
+    out = tmp_path / "dump"
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "0", "--batch", "1", "--hessian-nt", "0",
+           "--cfg1", "0", "--cfg5", "0", "--cfg4-seeds", "0", "--no-cpu-baseline", "--dump-outputs", str(out)]
+    p = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=str(tmp_path))
+    assert p.returncode == 0, p.stderr[-3000:]
+    line = json.loads(p.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 1
+    d = {f[:-4]: np.load(out / f) for f in os.listdir(out)}
+    assert sorted(d) == ["cost", "divT", "fidelities", "gradient", "psi_bond_dims", "xi_bond_dims"]
+    assert all(a.dtype == np.float64 for a in d.values())
+    z = load_golden("golden_cfg2_eval.npz")
+    assert d["cost"][0] == line["result"]["cost"]
+    assert abs(d["cost"][0] - float(z["cost"])) / abs(float(z["cost"])) < 1e-9
+    assert np.max(np.abs(d["gradient"] - z["grad"])) / np.max(np.abs(z["grad"])) < 1e-7
+    divT = d["divT"][:, 0] + 1j * d["divT"][:, 1]
+    assert np.max(np.abs(divT - z["divT"])) / np.max(np.abs(z["divT"])) < 1e-7
+    assert np.max(np.abs(d["fidelities"] - z["fidelities"])) < 1e-9
+    assert np.array_equal(d["psi_bond_dims"], z["psi_dims"])
+    assert np.array_equal(d["xi_bond_dims"], z["xi_dims"])
+
+
 @pytest.mark.parametrize("L,Np,chi,cutoff", [(30, 30, 150, 1e-8), (50, 50, 256, 1e-10)])
 def test_cfg4_cfg5_shapes_one_step(L, Np, chi, cutoff):
     """BASELINE.json configs[3] (L=30, chi=150) and configs[4] (L=50, chi=256, Cutoff 1e-10) at their full shapes: one forward
