@@ -14,6 +14,7 @@
 //      until every Gram entry <r_p|r_q> vanishes; one half-warp per pair, dot products by shuffles;
 //      the Gram diagonal (squared norms) is the spectrum the truncation rule sees
 //      -- jacobi_rot_kernel (rows register resident, jacobi_sweep_blocked) for blocks with at most 64 rows of R,
+//      (jacobi_rows_cluster_kernel: the same spread over a 4-CTA cluster by row blocks from 40 rows of R on, for calls with one or two chains),
 //      the generic loops at the end of jacobi_blocks_kernel otherwise;
 //   3. global truncation over all blocks (truncate_kernel);
 //   4. only the kept left vectors are formed, u_j = M z_j^H / |M z_j^H| (build_factors_kernel; for gauge moves it
@@ -1165,29 +1166,32 @@ __device__ bool gram_chol_block(const DecompArgs& a, const DecompBuffers& b, con
   return true;
 }
 
+// Rows of R handed over for the register-resident second stage by jacobi_blocks_kernel<true, true>, or -1 if the block is not
+// finished by that stage.  Only blocks of the register-cached first stage hand over to it; the hand-over entries of the others
+// may still be in the making on the cluster stream (launch_jacobi_blocks), so they are told apart by their shape.
+__device__ __forceinline__ int rot_handover_rows(const DecompBuffers& b, int blk, int smem_elems) {
+  const DecompWork* w = b.dw;
+  if (blk >= w->nblocks) return -1;
+  const int nv0 = w->blk[blk].nv, len0 = w->blk[blk].len;
+  const bool fits = nv0 * len0 <= smem_elems && nv0 <= JAC_NV_SMEM;
+  const int ldpad = ((nv0 + 15) >> 4) << 4;
+  const bool can_cache = nv0 <= 16 * JAC_EPL && (nv0 < len0 ? nv0 : len0) * ldpad <= smem_elems;
+  if (!(fits && can_cache)) return -1;
+  return reinterpret_cast<const int*>(b.scratch_d + 7 * NV_MAX + OCMPS_MAX_BLK)[blk];
+}
+
 // Second half of the block decomposition for the blocks handed over by jacobi_blocks_kernel<true, true>: one-sided
 // Jacobi on the rows of R with the rows held in registers (jacobi_sweep_blocked), then spectrum and right vectors.
-__global__ void __launch_bounds__(JAC_THREADS) jacobi_rot_kernel(DecompArgs a, DecompBuffers b, int smem_elems) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
+// One CTA of JAC_THREADS per block (block `blk`, keff rows of R).
+__device__ __forceinline__ void jacobi_rot_block(const DecompArgs& a, const DecompBuffers& b, int blk, int keff, unsigned char* smem_raw) {
   __shared__ int s_rot, s_big;
   __shared__ double s_nrm[JAC_BLOCKED_ROWS];
   const DecompWork* w = b.dw;
-  if ((int)blockIdx.x >= w->nblocks) return;
-  {   // only blocks of the register-cached first stage hand over to this kernel; the hand-over entries of the others may still be
-      // in the making on the cluster stream (launch_jacobi_blocks), so they are told apart by their shape
-    const int nv0 = w->blk[blockIdx.x].nv, len0 = w->blk[blockIdx.x].len;
-    const bool fits = nv0 * len0 <= smem_elems && nv0 <= JAC_NV_SMEM;
-    const int ldpad = ((nv0 + 15) >> 4) << 4;
-    const bool can_cache = nv0 <= 16 * JAC_EPL && (nv0 < len0 ? nv0 : len0) * ldpad <= smem_elems;
-    if (!(fits && can_cache)) return;
-  }
-  const int keff = reinterpret_cast<const int*>(b.scratch_d + 7 * NV_MAX + OCMPS_MAX_BLK)[blockIdx.x];
-  if (keff < 0) return;                                   // finished by the first kernel
-  const DecompBlock B = w->blk[blockIdx.x];
+  const DecompBlock B = w->blk[blk];
   const int nv = B.nv;
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = JAC_THREADS / 32;
   const int epl = (nv + 15) >> 4, ldz = epl << 4;
-  const double F = (b.scratch_d + 7 * NV_MAX)[blockIdx.x];
+  const double F = (b.scratch_d + 7 * NV_MAX)[blk];
   const double thr = F * DEFLATE_REL;
   const short* perm = reinterpret_cast<const short*>(b.scratch_d + 4 * NV_MAX) + B.p_off;
   cplx* Ya = b.ywork + B.ws_off;
@@ -1234,7 +1238,7 @@ __global__ void __launch_bounds__(JAC_THREADS) jacobi_rot_kernel(DecompArgs a, D
       atomicAdd(&g_jac_dbg[7], (unsigned long long)(t_jac1 - t_jac0));
     }
 #ifdef OCMPS_JAC_TRACE
-    if (nv >= 24) printf("JT2 kind %d blk %d nv %d keff %d jac %lld\n", a.kind, (int)blockIdx.x, nv, keff, t_jac1 - t_jac0);
+    if (nv >= 24) printf("JT2 kind %d blk %d nv %d keff %d jac %lld\n", a.kind, blk, nv, keff, t_jac1 - t_jac0);
 #endif
   }
   // spectrum + normalised right vectors Z[j][physical vector]
@@ -1254,6 +1258,13 @@ __global__ void __launch_bounds__(JAC_THREADS) jacobi_rot_kernel(DecompArgs a, D
       b.P[B.p_off + v] = 0.0;
     }
   }
+}
+
+__global__ void __launch_bounds__(JAC_THREADS) jacobi_rot_kernel(DecompArgs a, DecompBuffers b, int smem_elems) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int keff = rot_handover_rows(b, (int)blockIdx.x, smem_elems);
+  if (keff < 0) return;                                   // not handed over to this stage
+  jacobi_rot_block(a, b, (int)blockIdx.x, keff, smem_raw);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1832,6 +1843,265 @@ __global__ void __launch_bounds__(BJ_THREADS) jacobi_big_kernel(DecompArgs a, De
 }
 
 // ------------------------------------------------------------------------------------------------
+// Register-cached blocks with many rows of R: row-block parallel Jacobi on a cluster of RC_C CTAs
+// ------------------------------------------------------------------------------------------------
+// The largest block of a saturated gate decomposition (nv ~ 80, ~62 rows of R) sets the latency of the whole decomposition, and
+// on one SM a rotation round of jacobi_sweep_blocked is bound by that SM's instruction issue (16 warps, 4 per scheduler), not by
+// the round's dependent chain (profiles/r02_cluster_jacobi.md).  Here the rows are split into RC_NBLK = 2 RC_C row blocks of
+// rb = ceil(keff / RC_NBLK) <= 8 rows and every CTA of the cluster holds two of them, so dot products and rotations stay local
+// and every SM carries a quarter of the issue load.  A sweep = the pairs inside every row block, then RC_NBLK - 1 block rounds
+// of a round-robin tournament over the row blocks; in a block round a CTA does the rb x rb cross pairs of its two blocks in rb
+// rotation rounds (one half-warp per row of the first block, rows of the second one passed on through shared memory).
+// Between block rounds every CTA pulls the two blocks of its next pairing from the CTAs that held them (ld.shared::cluster,
+// double-buffered, one cluster barrier per block round).  The round-robin does not let a CTA keep one of its blocks in every
+// transition, so both are always pulled (the one it keeps from itself); that is ~2 x 10 KB per CTA per block round.
+// The stop flags are OR-reduced over the cluster once per sweep, so every CTA applies the same stop rule and the result is
+// deterministic (fixed pair order); it is not bitwise that of jacobi_rot_kernel (the rotation order differs).
+constexpr int RC_C = 4;                                    // CTAs per cluster
+constexpr int RC_NBLK = 2 * RC_C;                          // row blocks of the tournament
+constexpr int RC_ROWS = JAC_BLOCKED_ROWS / RC_NBLK;        // rows per row block, at most
+constexpr int RC_WORK_THREADS = 16 * RC_ROWS;              // one half-warp per row of a block
+// blocks with at least this many rows of R take the cluster path (K_CL); smaller ones stay with jacobi_rot_block on one SM
+constexpr int RC_MIN_ROWS = 40;
+
+__device__ unsigned long long g_rc_dbg[2];                 // development counters: [0] blocks finished on the cluster path, [1] their sweeps
+
+struct RcShared {
+  double nrm[2][2][RC_ROWS];       // cached squared norms: [buffer][block of this CTA][row]
+  int flags[2][RC_C];              // per sweep parity and rank: rotated | (rotated above 1e-8) << 1
+  int rot, big;
+};
+
+// the two row blocks CTA s plays in block round R (round-robin over RC_NBLK blocks with RC_C pair slots)
+__device__ __forceinline__ void rc_blocks(int R, int s, int& P, int& Q) {
+  constexpr int mm = RC_NBLK - 1;
+  int p = R + s; if (p >= mm) p -= mm;
+  int q = R - s; if (q < 0) q += mm;
+  if (s == 0) q = RC_NBLK - 1;
+  P = p; Q = q;
+}
+
+__device__ __forceinline__ void rc_bar() { asm volatile("bar.sync 1, %0;" ::"n"(RC_WORK_THREADS) : "memory"); }
+
+// One block round of the RC_WORK_THREADS working threads: (intra: the pairs inside both blocks first) the rb x rb cross pairs of
+// block 0 (rows Z0, norms n0, global rows base0 + i) and block 1.  Rows past keff are zero padding and take no part.
+template <int EPL>
+__device__ __forceinline__ void rc_block_round(cplx* __restrict__ Z0, cplx* __restrict__ Z1, double* n0, double* n1, int rb, int base0, int base1,
+                                               int keff, double thr, bool intra, int* s_rot, int* s_big) {
+  constexpr int ldz = 16 * EPL;
+  const int tid = threadIdx.x, hl = tid & 15, h = tid >> 4;
+  cplx ra[EPL], rb_[EPL];
+  double na = 0.0, nb = 0.0;
+  auto load_row = [&](cplx (&r)[EPL], double& n, const cplx* Z, const double* nz, int row) {
+    const cplx* z = Z + (row >= 0 ? row : 0) * ldz + hl;
+#pragma unroll
+    for (int e = 0; e < EPL; ++e) r[e] = row >= 0 ? z[16 * e] : make_double2(0.0, 0.0);
+    n = row >= 0 ? nz[row] : 0.0;
+  };
+  auto store_row = [&](const cplx (&r)[EPL], double n, cplx* Z, double* nz, int row) {
+    cplx* z = Z + row * ldz + hl;
+#pragma unroll
+    for (int e = 0; e < EPL; ++e) z[16 * e] = r[e];
+    if (hl == 0) nz[row] = n;
+  };
+  if (intra) {   // half-warps [0, RC_ROWS/2) take the pairs of block 0, the others those of block 1; round-robin over rbp rows
+    const int X = h / (RC_ROWS / 2), j = h % (RC_ROWS / 2);
+    cplx* Z = X ? Z1 : Z0;
+    double* nz = X ? n1 : n0;
+    const int base = X ? base1 : base0;
+    const int rbp = (rb + 1) & ~1, m = rbp - 1;
+    for (int r = 0; r < m; ++r) {
+      int p = r + j; if (p >= m) p -= m;
+      int q = r - j; if (q < 0) q += m;
+      if (j == 0) q = m;
+      const bool act = 2 * j < rbp && p < rb && q < rb && base + p < keff && base + q < keff;
+      load_row(ra, na, Z, nz, act ? p : -1);
+      load_row(rb_, nb, Z, nz, act ? q : -1);
+      jac_rotate<EPL>(ra, rb_, na, nb, act, thr, hl, s_rot, s_big);
+      if (act) { store_row(ra, na, Z, nz, p); store_row(rb_, nb, Z, nz, q); }
+      rc_bar();
+    }
+  }
+  // cross pairs: half-warp h keeps row h of block 0 in registers and meets row (h + t) mod rb of block 1 in round t
+  const bool has_a = h < rb && base0 + h < keff;
+  load_row(ra, na, Z0, n0, has_a ? h : -1);
+  for (int t = 0; t < rb; ++t) {
+    int jb = h + t; if (jb >= rb) jb -= rb;
+    const bool act = has_a && base1 + jb < keff;
+    load_row(rb_, nb, Z1, n1, act ? jb : -1);
+    jac_rotate<EPL>(ra, rb_, na, nb, act, thr, hl, s_rot, s_big);
+    if (act) store_row(rb_, nb, Z1, n1, jb);
+    rc_bar();
+  }
+  if (has_a) store_row(ra, na, Z0, n0, h);
+}
+
+template <int EPL>
+__device__ __forceinline__ void rc_run(const DecompArgs& a, const DecompBuffers& b, int blk, int keff, unsigned rank, cplx* __restrict__ Zs, RcShared& sh) {
+  constexpr int ldz = 16 * EPL;
+  constexpr int BLK = RC_ROWS * ldz;                     // elements of one row block in a buffer
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = JAC_THREADS / 32;
+  const DecompBlock B = b.dw->blk[blk];
+  const int nv = B.nv;
+  const int rb = (keff + RC_NBLK - 1) / RC_NBLK;
+  const double F = (b.scratch_d + 7 * NV_MAX)[blk];
+  const double thr = F * DEFLATE_REL;
+  const cplx* Yb = b.ywork + b.ywork_half + B.ws_off;   // R, keff rows of stride ldz (the padding of a row is zero)
+  auto zb = [&](int buf, int k) { return Zs + (2 * buf + k) * BLK; };
+  const long long t_jac0 = clock64();
+  int P, Q;
+  rc_blocks(0, (int)rank, P, Q);
+  for (int e = tid; e < 2 * BLK; e += JAC_THREADS) {
+    const int k = e / BLK, r = (e % BLK) / ldz, c = e % ldz;
+    const int row = (k ? Q : P) * rb + r;
+    Zs[e] = (r < rb && row < keff) ? Yb[row * ldz + c] : make_double2(0.0, 0.0);
+  }
+  __syncthreads();
+  int cur = 0;
+  bool done = false;
+#ifdef OCMPS_JAC_TRACE
+  long long t_work = 0, t_xchg = 0;
+  int nrounds = 0, nxchg = 0;
+#endif
+  for (int sweep = 0; sweep < JAC_MAX_SWEEPS && !done; ++sweep) {
+    for (int lr = warp; lr < 2 * RC_ROWS; lr += nwarps) {     // exact Gram diagonal at the start of every sweep
+      const int k = lr / RC_ROWS, r = lr % RC_ROWS;
+      const cplx* y = zb(cur, k) + r * ldz;
+      double s = 0.0;
+      for (int c = lane; c < nv; c += 32) { const cplx u = y[c]; s += u.x * u.x + u.y * u.y; }
+      s = warp_sum(s);
+      if (lane == 0) sh.nrm[cur][k][r] = s;                   // (zero for padding rows)
+    }
+    if (tid == 0) { sh.rot = 0; sh.big = 0; }
+    __syncthreads();
+    for (int R = 0; R < RC_NBLK - 1; ++R) {
+#ifdef OCMPS_JAC_TRACE
+      const long long tw0 = clock64();
+#endif
+      if (tid < RC_WORK_THREADS) rc_block_round<EPL>(zb(cur, 0), zb(cur, 1), sh.nrm[cur][0], sh.nrm[cur][1], rb, P * rb, Q * rb, keff, thr, R == 0, &sh.rot, &sh.big);
+      __syncthreads();
+#ifdef OCMPS_JAC_TRACE
+      const long long tw1 = clock64();
+      t_work += tw1 - tw0;
+      nrounds += rb + (R == 0 ? ((rb + 1) & ~1) - 1 : 0);
+#endif
+      const bool last = R == RC_NBLK - 2;
+      if (last && tid < RC_C) {     // this CTA's flags into slot `rank` of every CTA (released by the cluster barrier)
+        const int f = (sh.rot ? 1 : 0) | (sh.big ? 2 : 0);
+        asm volatile("st.shared::cluster.u32 [%0], %1;" ::"r"(clus::mapa(clus::smem_u32(&sh.flags[sweep & 1][rank]), (unsigned)tid)), "r"(f) : "memory");
+      }
+      clus::cluster_sync();
+      if (last) {
+        int any = 0;
+#pragma unroll
+        for (int r = 0; r < RC_C; ++r) any |= sh.flags[sweep & 1][r];
+        // quadratic convergence: if every rotated pair had |<p|q>| < 1e-8 |p||q|, the residuals are now ~1e-16
+        done = !(any & 1) || !(any & 2);
+        if (tid == 0 && rank == 0) {
+          atomicAdd(&g_jac_dbg[0], 1ull); atomicMax(&g_jac_dbg[2], (unsigned long long)(sweep + 1)); atomicAdd(&g_rc_dbg[1], 1ull);
+          if (nv >= 64) atomicAdd(&g_jac_dbg[3], 1ull);
+          if (nv >= 64 && sweep == 0) atomicAdd(&g_jac_dbg[4], 1ull);
+          if (!done && sweep == JAC_MAX_SWEEPS - 1) atomicOr(b.status, OCMPS_ST_NOCONV);
+        }
+        if (done || sweep == JAC_MAX_SWEEPS - 1) break;
+      }
+      // pull the two blocks of the next pairing (round 0 of the next sweep after the last round) from the CTAs that hold them
+      // (the one this CTA keeps from itself)
+      int NP, NQ;
+      rc_blocks(last ? 0 : R + 1, (int)rank, NP, NQ);
+      unsigned src0 = 0, src1 = 0, nsrc0 = 0, nsrc1 = 0;       // shared::cluster addresses of their rows / norms
+      for (int s = 0; s < RC_C; ++s) {
+        int p, q;
+        rc_blocks(R, s, p, q);
+        const unsigned zp = clus::mapa(clus::smem_u32(zb(cur, 0)), (unsigned)s), zq = clus::mapa(clus::smem_u32(zb(cur, 1)), (unsigned)s);
+        const unsigned np = clus::mapa(clus::smem_u32(sh.nrm[cur][0]), (unsigned)s), nq = clus::mapa(clus::smem_u32(sh.nrm[cur][1]), (unsigned)s);
+        if (p == NP) { src0 = zp; nsrc0 = np; }
+        if (q == NP) { src0 = zq; nsrc0 = nq; }
+        if (p == NQ) { src1 = zp; nsrc1 = np; }
+        if (q == NQ) { src1 = zq; nsrc1 = nq; }
+      }
+      for (int e = tid; e < 2 * rb * ldz; e += JAC_THREADS) {
+        const int k = e >= rb * ldz, o = e - k * rb * ldz;
+        double xr, xi;
+        asm volatile("ld.shared::cluster.v2.f64 {%0, %1}, [%2];" : "=d"(xr), "=d"(xi) : "r"((k ? src1 : src0) + (unsigned)o * 16u) : "memory");
+        zb(cur ^ 1, k)[o] = make_double2(xr, xi);
+      }
+      if (tid < 2 * RC_ROWS) {
+        const int k = tid / RC_ROWS, r = tid % RC_ROWS;
+        double x;
+        asm volatile("ld.shared::cluster.f64 %0, [%1];" : "=d"(x) : "r"((k ? nsrc1 : nsrc0) + (unsigned)r * 8u) : "memory");
+        sh.nrm[cur ^ 1][k][r] = x;
+      }
+      __syncthreads();
+#ifdef OCMPS_JAC_TRACE
+      t_xchg += clock64() - tw1;
+      ++nxchg;
+#endif
+      cur ^= 1; P = NP; Q = NQ;
+    }
+  }
+  const long long t_jac1 = clock64();
+  // spectrum + normalised right vectors Z[j][physical vector]: every CTA writes the rows it holds
+  const short* perm = reinterpret_cast<const short*>(b.scratch_d + 4 * NV_MAX) + B.p_off;
+  cplx* Ya = b.ywork + B.ws_off;
+  for (int lr = warp; lr < 2 * RC_ROWS; lr += nwarps) {
+    const int k = lr / RC_ROWS, r = lr % RC_ROWS, v = (k ? Q : P) * rb + r;
+    if (r >= rb || v >= keff) continue;
+    const cplx* y = zb(cur, k) + r * ldz;
+    double s = 0.0;
+    for (int c = lane; c < nv; c += 32) { const cplx u = y[c]; s += u.x * u.x + u.y * u.y; }
+    s = warp_sum(s);
+    const double inv = s > 0.0 ? rsqrt(s) : 0.0;
+    for (int c = lane; c < nv; c += 32) {
+      const cplx u = y[c];
+      Ya[v * nv + (int)perm[c]] = make_double2(u.x * inv, u.y * inv);
+    }
+    if (lane == 0) b.P[B.p_off + v] = s;
+  }
+  if (rank == 0) for (int v = keff + tid; v < nv; v += JAC_THREADS) b.P[B.p_off + v] = 0.0;
+  if (tid == 0 && rank == 0) {
+    atomicAdd(&g_jac_dbg[1], 1ull);
+    atomicAdd(&g_rc_dbg[0], 1ull);
+    if (nv >= 64) {
+      atomicAdd(&g_jac_dbg[6], (unsigned long long)(t_jac1 - t_jac0));
+      atomicAdd(&g_jac_dbg[7], (unsigned long long)(t_jac1 - t_jac0));
+    }
+#ifdef OCMPS_JAC_TRACE
+    if (nv >= 24)
+      printf("JTR kind %d blk %d nv %d keff %d rb %d jac %lld : rotation rounds %d, %lld clk per round; block exchanges %d, %lld clk each\n", a.kind, blk, nv,
+             keff, rb, t_jac1 - t_jac0, nrounds, nrounds ? t_work / nrounds : 0ll, nxchg, nxchg ? t_xchg / nxchg : 0ll);
+#endif
+  }
+  // (no DSMEM access follows the last cluster barrier: a CTA may leave while its peers write their rows)
+}
+
+// Second stage of the register-cached blocks, one cluster of RC_C CTAs per block: blocks with at least RC_MIN_ROWS rows of R are
+// spread over the cluster (rc_run), smaller ones are finished by rank 0 alone (jacobi_rot_block) while the other ranks leave.
+__global__ void __launch_bounds__(JAC_THREADS) jacobi_rows_cluster_kernel(DecompArgs a, DecompBuffers b, int smem_elems) {
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  __shared__ RcShared sh;
+  const int blk = (int)blockIdx.x / RC_C;
+  const unsigned rank = clus::cluster_rank();
+  const int keff = rot_handover_rows(b, blk, smem_elems);   // (uniform over the cluster)
+  if (keff < 0) return;
+  if (keff < RC_MIN_ROWS) {
+    if (rank == 0) jacobi_rot_block(a, b, blk, keff, smem_raw);
+    return;
+  }
+  cplx* Zs = reinterpret_cast<cplx*>(smem_raw);
+  switch ((b.dw->blk[blk].nv + 15) >> 4) {
+    case 1: rc_run<1>(a, b, blk, keff, rank, Zs, sh); break;
+    case 2: rc_run<2>(a, b, blk, keff, rank, Zs, sh); break;
+    case 3: rc_run<3>(a, b, blk, keff, rank, Zs, sh); break;
+    case 4: rc_run<4>(a, b, blk, keff, rank, Zs, sh); break;
+    case 5: rc_run<5>(a, b, blk, keff, rank, Zs, sh); break;
+    case 6: rc_run<6>(a, b, blk, keff, rank, Zs, sh); break;
+    case 7: rc_run<7>(a, b, blk, keff, rank, Zs, sh); break;
+    default: rc_run<8>(a, b, blk, keff, rank, Zs, sh); break;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // global truncation (ITensor truncate(), SURVEY A.3) + new bond bookkeeping + follow-up descriptor
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(1024) truncate_kernel(DecompArgs a, DecompBuffers b, TruncParams tp) {
@@ -2270,6 +2540,11 @@ void debug_jacobi_counters(unsigned long long* out, bool reset) {
   if (reset) { unsigned long long z[8] = {0}; cudaMemcpyToSymbol(g_jac_dbg, z, sizeof(z)); }
 }
 
+void debug_row_cluster_counters(unsigned long long* out, bool reset) {
+  cudaMemcpyFromSymbol(out, g_rc_dbg, sizeof(unsigned long long) * 2);
+  if (reset) { unsigned long long z[2] = {0, 0}; cudaMemcpyToSymbol(g_rc_dbg, z, sizeof(z)); }
+}
+
 // von Neumann entropy of the spectrum the last decomposition left in b.P (include/correlations.hpp:119-148):
 // S = -sum_{p > 1e-12} p ln p over the squared singular values of all charge blocks.  One CTA, fixed-order tree.
 __global__ void __launch_bounds__(256) spectrum_entropy_kernel(DecompBuffers b, double* out) {
@@ -2326,7 +2601,8 @@ void profile_read(double* out) {
 }
 
 void launch_jacobi_blocks(const DecompArgs& a, const DecompBuffers& b, int nblk_launch, size_t smem_limit, bool need_global,
-                          bool long_rows, double rank_tol, int max_rows, int capV, int capC, cudaStream_t s, const SvdFork* fork) {
+                          bool long_rows, double rank_tol, int max_rows, int capV, int capC, bool spread_rows, cudaStream_t s,
+                          const SvdFork* fork) {
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (g_prof_on) {
     if (g_prof_used == g_prof_events.size()) {
@@ -2349,6 +2625,7 @@ void launch_jacobi_blocks(const DecompArgs& a, const DecompBuffers& b, int nblk_
     cudaFuncSetAttribute(jacobi_blocks_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
     cudaFuncSetAttribute(build_factors_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
     cudaFuncSetAttribute(jacobi_rot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(JAC_BLOCKED_ROWS * 16 * JAC_EPL * sizeof(cplx)));
+    cudaFuncSetAttribute(jacobi_rows_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(JAC_BLOCKED_ROWS * 16 * JAC_EPL * sizeof(cplx)));
     cudaFuncSetAttribute(jacobi_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(BJ_MAX_ROWS * (BJ_TPP * BJ_MAX_EPL + 4) * sizeof(cplx)));
     cudaFuncSetAttribute(qr_big_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)((32 * BJ_MAX_ROWS + BJ_MAX_ROWS) * sizeof(cplx)));
     g_jac_attr_set[dev] = true;
@@ -2389,7 +2666,20 @@ void launch_jacobi_blocks(const DecompArgs& a, const DecompBuffers& b, int nblk_
     cfg.attrs = at; cfg.numAttrs = 1;
     cudaLaunchKernelEx(&cfg, qr_big_kernel, a, b, (int)(smem_limit / sizeof(cplx)), rank_tol);
   }
-  jacobi_rot_kernel<<<nblk_launch, JAC_THREADS, JAC_BLOCKED_ROWS * 16 * JAC_EPL * sizeof(cplx), s>>>(a, b, (int)(smem_limit / sizeof(cplx)));
+  if (spread_rows) {   // second stage of the register-cached blocks: one cluster per block, spread over it from RC_MIN_ROWS rows of R on
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(nblk_launch * RC_C, 1, 1);
+    cfg.blockDim = dim3(JAC_THREADS, 1, 1);
+    cfg.dynamicSmemBytes = (size_t)JAC_BLOCKED_ROWS * 16 * JAC_EPL * sizeof(cplx);
+    cfg.stream = s;
+    cudaLaunchAttribute at[1];
+    at[0].id = cudaLaunchAttributeClusterDimension;
+    at[0].val.clusterDim.x = RC_C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+    cfg.attrs = at; cfg.numAttrs = 1;
+    cudaLaunchKernelEx(&cfg, jacobi_rows_cluster_kernel, a, b, (int)(smem_limit / sizeof(cplx)));
+  } else {
+    jacobi_rot_kernel<<<nblk_launch, JAC_THREADS, JAC_BLOCKED_ROWS * 16 * JAC_EPL * sizeof(cplx), s>>>(a, b, (int)(smem_limit / sizeof(cplx)));
+  }
   if (big_on & 1) {
     if (forked) cudaStreamWaitEvent(sb, fork->ev_first, 0);
     cudaLaunchConfig_t cfg = {};

@@ -150,6 +150,10 @@ struct Workspace {
   // Third stream: inside one decomposition the blocks that fit one SM (QR -> register-resident rotations) and the blocks that
   // need a cluster (qr_big -> jacobi_big) are independent chains of kernels; the cluster chain runs on `side2` beside the other.
   SvdFork fork;
+  // Second stage of the largest register-cached charge blocks spread over a thread-block cluster (jacobi_rows_cluster_kernel):
+  // set per call by WsLease::acquire, for calls that run one or two chains.  With many chains in flight every SM is busy anyway
+  // and four SMs per block would cost throughput, so those calls keep the one-SM kernel.
+  bool spread_jacobi = true;
   // overlaps
   cplx* E[2] = {nullptr, nullptr};
   cplx* T = nullptr;
@@ -167,9 +171,9 @@ struct Workspace {
   ocmps_mps* psiH = nullptr;        // Hessian-row state of this chain
   ocmps_store* rowstore = nullptr;  // Hessian rows: the last few propagated slices, overlapped with xiH in one batched pass
   // CUDA graphs of one Trotter step (+ slice store), keyed by stepper serial, MPS serial, buffer parity, with/without
-  // store, and the block-grid bound (ctx->qmax) that the launches of the captured sequence were sized with
+  // store, the block-grid bound (ctx->qmax) that the launches of the captured sequence were sized with, and spread_jacobi
   struct StepGraph { cudaGraphExec_t exec = nullptr; unsigned long long flips = 0; int launches = 0; int seen = 0; };
-  std::map<std::tuple<long long, long long, unsigned long long, int, int>, StepGraph> graphs;
+  std::map<std::tuple<long long, long long, unsigned long long, int, int, int>, StepGraph> graphs;
 };
 
 struct ocmps_stepper {
@@ -362,6 +366,7 @@ struct WsLease {
       c->pool.push_back(w);
       ws.push_back(w);
     }
+    for (Workspace* w : ws) w->spread_jacobi = n <= 2;
     for (Workspace* w : ws) {          // graphs of MPS destroyed since this workspace was last used
       if (w->dead_seen == c->dead_mps.size()) continue;
       if (!w->graphs.empty()) {
@@ -551,7 +556,7 @@ void run_decomp(Workspace* ws, const DecompArgs& a, const TruncParams& tp, int c
   rank_tol = std::min(rank_scale * 1e-8, std::max(1e-30, rank_tol));
   const bool long_rows = capV > 128;                   // rows of R longer than the register-cached path handles
   const int max_rows = std::min(capV, capC);           // rows of R of the largest possible block
-  launch_jacobi_blocks(a, db, nblk, smem, need_global, long_rows, rank_tol, max_rows, capV, capC, s, &ws->fork);
+  launch_jacobi_blocks(a, db, nblk, smem, need_global, long_rows, rank_tol, max_rows, capV, capC, ws->spread_jacobi, s, &ws->fork);
   g_trace.mark((a.kind == DK_GATE_LEFT || a.kind == DK_GATE_RIGHT) ? TR_SVD_GATE : TR_SVD_ORTH, s);
   launch_truncate(a, db, tp, s);
   g_trace.mark(TR_TRUNC, s);
@@ -779,7 +784,7 @@ int step_enqueue(ocmps_stepper* st, ocmps_mps* m, Workspace* ws, double from, do
   if (!graphs_enabled() || profile_is_on()) { body(); return OCMPS_OK; }   // event timing needs plain launches
   unsigned long long parity = 0;
   for (int j = 0; j < lay.L; ++j) parity |= (unsigned long long)(m->cur[j] & 1) << j;
-  auto key = std::make_tuple(st->serial, m->serial, parity, store ? 1 : 0, ws->ctx->qmax.load());
+  auto key = std::make_tuple(st->serial, m->serial, parity, store ? 1 : 0, ws->ctx->qmax.load(), ws->spread_jacobi ? 1 : 0);
   Workspace::StepGraph& g = ws->graphs[key];
   if (g.exec) {
     for (int j = 0; j < lay.L; ++j) m->cur[j] ^= (int)((g.flips >> j) & 1ull);
@@ -925,6 +930,7 @@ int apply_K_async(ocmps_stepper* st, Workspace* ws, ocmps_mps* in, ocmps_mps* ou
   }
   ocmps_mps* big = ws->big;
   Workspace* bw = ws->bigws;
+  bw->spread_jacobi = ws->spread_jacobi;
   const Layout& lb = big->lay;
   if (L == 1) return fail(OCMPS_ERR_INVALID, "apply_K needs L >= 2");
   for (int j = 0; j < L; ++j) big->cur[j] = 0;
@@ -1333,6 +1339,8 @@ int ocmps_step(ocmps_stepper* st, ocmps_mps* psi, double from, double to, int fo
 }
 
 int ocmps_debug_jacobi(unsigned long long* out, int reset) { cudaDeviceSynchronize(); debug_jacobi_counters(out, reset != 0); return 0; }
+// out[0]: charge blocks whose Jacobi stage ran spread over a thread-block cluster (row-block path), out[1]: their sweeps
+int ocmps_debug_row_cluster(unsigned long long* out2, int reset) { cudaDeviceSynchronize(); debug_row_cluster_counters(out2, reset != 0); return 0; }
 
 // development aid: run ops [op_begin, op_end) of one step (not part of include/ocmps.h)
 int ocmps_debug_run_ops(ocmps_stepper* st, ocmps_mps* psi, double from, double to, int forward, int op_begin, int op_end) {

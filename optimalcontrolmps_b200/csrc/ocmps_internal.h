@@ -73,6 +73,7 @@ struct Phases { double re[4][OCMPS_MAX_D]; double im[4][OCMPS_MAX_D]; };
 extern std::atomic<long long> g_ocmps_launches;   // kernels launched so far (bench.py reports it)
 
 void debug_jacobi_counters(unsigned long long* out, bool reset);
+void debug_row_cluster_counters(unsigned long long* out, bool reset);
 void profile_enable(bool on);
 bool profile_is_on();
 void profile_read(double* out);
@@ -119,7 +120,8 @@ void launch_decomp_setup(const DecompArgs& a, const DecompBuffers& b, cudaStream
 // second stream + events for the cluster chain of a decomposition (qr_big -> jacobi_big beside QR -> rotations), see decomp.cu
 struct SvdFork { cudaStream_t stream = nullptr; cudaEvent_t ev_fork = nullptr, ev_first = nullptr, ev_join = nullptr; };
 void launch_jacobi_blocks(const DecompArgs& a, const DecompBuffers& b, int nblk_launch, size_t smem_limit, bool need_global,
-                          bool long_rows, double rank_tol, int max_rows, int capV, int capC, cudaStream_t s, const SvdFork* fork = nullptr);
+                          bool long_rows, double rank_tol, int max_rows, int capV, int capC, bool spread_rows, cudaStream_t s,
+                          const SvdFork* fork = nullptr);
 void launch_spectrum_entropy(const DecompBuffers& b, double* out, cudaStream_t s);
 void launch_truncate(const DecompArgs& a, const DecompBuffers& b, const TruncParams& tp, cudaStream_t s);
 void launch_build_factors(const DecompArgs& a, const DecompBuffers& b, int cap_k, int cap_vec, int cap_comp, cudaStream_t s);
