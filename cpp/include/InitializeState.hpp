@@ -26,5 +26,24 @@ inline IQMPS InitializeState(const SiteSet& sites, const int Npart, const double
   return InitializeState(sites, Npart, J, U, 200, 1E-9, silent);          // :52-54
 }
 
+// The same ground state by two-site DMRG on the device, the algorithm of the reference (10 sweeps, maxm 10, 20, 50, maxBondDim,
+// cutoff `threshold`; no noise term): ocmps_ground_state_dmrg.
+inline IQMPS InitializeStateDMRG(const SiteSet& sites, const int Npart, const double J, const double U, const int maxBondDim,
+                                 const double threshold, bool silent = true) {
+  (void)silent;
+  const int L = sites.N(), D = sites.D();
+  long long full = 1;
+  for (int i = 0; i < L / 2 && full < 4096; ++i) full *= D;
+  const int cap = (int)std::min<long long>(maxBondDim, full);
+  IQMPS psi(L, D, cap);
+  ocmps_check(ocmps_ground_state_dmrg(default_context(), L, D, Npart, J, U, cap, threshold, 10, psi.handle(), nullptr, nullptr),
+              "ocmps_ground_state_dmrg");
+  return psi;
+}
+
+inline IQMPS InitializeStateDMRG(const SiteSet& sites, const int Npart, const double J, const double U, bool silent = true) {
+  return InitializeStateDMRG(sites, Npart, J, U, 200, 1E-9, silent);
+}
+
 }  // namespace itensor
 #endif

@@ -101,6 +101,13 @@ int ocmps_stepper_gate(ocmps_stepper* st, int forward, double* out);
  * normalised with its orthogonality centre at site 1.  energy / steps may be NULL. */
 int ocmps_ground_state(ocmps_ctx* ctx, int L, int D, int Npart, double J, double U, int maxm, double cutoff, double tau_final,
                        ocmps_mps* out, double* energy, int* steps);
+/* The same ground state by two-site DMRG on the device, as the reference computes it (include/InitializeState.hpp:18-117:
+ * `nsweeps` sweeps, maxm 10, 20, 50, maxm, cutoff; no noise term): the same start state, a Lanczos solve with 4 Krylov vectors
+ * at every bond, the engine's truncating decomposition.  `out` must have capacity >= maxm (maxm < 1 selects the capacity); it
+ * ends normalised with its orthogonality centre at site 1.  `energy` (may be NULL) is <psi|H|psi> of the returned state;
+ * `sweep_energies` (nsweeps entries, or NULL) the last Ritz value of every sweep. */
+int ocmps_ground_state_dmrg(ocmps_ctx* ctx, int L, int D, int Npart, double J, double U, int maxm, double cutoff, int nsweeps,
+                            ocmps_mps* out, double* energy, double* sweep_energies);
 
 /* ---- resident slice stores and sweeps (OptimalControl::calcPsi / calcXi / calcDivT) ---- */
 int ocmps_store_create(ocmps_ctx* ctx, int L, int D, int chi_cap, int nslots, ocmps_store** out);

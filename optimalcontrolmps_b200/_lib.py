@@ -18,7 +18,7 @@ SYMBOLS = [
     "ocmps_mps_create", "ocmps_mps_destroy", "ocmps_mps_upload", "ocmps_mps_sizes", "ocmps_mps_download",
     "ocmps_mps_bond_dims", "ocmps_mps_copy", "ocmps_mps_position1", "ocmps_mps_norm", "ocmps_overlap", "ocmps_overlap_K",
     "ocmps_stepper_create", "ocmps_stepper_destroy", "ocmps_stepper_set_tstep", "ocmps_stepper_get_tstep",
-    "ocmps_step", "ocmps_apply_K", "ocmps_ground_state", "ocmps_stepper_schedule", "ocmps_stepper_gate",
+    "ocmps_step", "ocmps_apply_K", "ocmps_ground_state", "ocmps_ground_state_dmrg", "ocmps_stepper_schedule", "ocmps_stepper_gate",
     "ocmps_store_create", "ocmps_store_destroy", "ocmps_store_get", "ocmps_store_put", "ocmps_store_bond_dims",
     "ocmps_forward_sweep", "ocmps_backward_sweep", "ocmps_sweep_pair", "ocmps_sweep_batch", "ocmps_backward_sweep_divT",
     "ocmps_store_overlaps", "ocmps_store_divT", "ocmps_store_apply_K", "ocmps_hessian_rows", "ocmps_hessian_eval",
@@ -94,6 +94,7 @@ def load():
         "ocmps_store_entanglement_entropy": (i, [vp, i, i, pd]),
         "ocmps_store_correlations": (i, [vp, i, pd, i, pi, i, pd]),
         "ocmps_ground_state": (i, [vp, i, i, i, d, d, i, d, d, vp, pd, pi]),
+        "ocmps_ground_state_dmrg": (i, [vp, i, i, i, d, d, i, d, i, vp, pd, pd]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

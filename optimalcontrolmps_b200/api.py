@@ -337,6 +337,23 @@ def InitializeState(sites: "BoseHubbard", Npart: int, J: float, U: float, maxBon
     return (out, e.value, n.value) if return_info else out
 
 
+def InitializeStateDMRG(sites: "BoseHubbard", Npart: int, J: float, U: float, maxBondDim: int = 200, threshold: float = 1e-9,
+                        nsweeps: int = 10, ctx: Optional["Context"] = None, chi_cap: Optional[int] = None, return_info: bool = False):
+    """The ground state of ``InitializeState`` computed as the reference computes it (include/InitializeState.hpp:18-117): two-site
+    DMRG on the device, ``nsweeps`` sweeps with maxm 10, 20, 50, maxBondDim and cutoff ``threshold``, no noise term
+    (``ocmps_ground_state_dmrg``).  Returns a DeviceMPS, or ``(psi, energy, sweep_energies)`` with ``return_info``: ``energy`` is
+    <psi|H|psi> of the returned state, ``sweep_energies`` the last Ritz value of every sweep."""
+    ctx = ctx or Context.default()
+    L, D = sites.N(), sites.D
+    cap = int(chi_cap or min(maxBondDim, D ** (L // 2)))
+    out = DeviceMPS(ctx, L, D, cap)
+    e = C.c_double()
+    sweeps = np.zeros(max(int(nsweeps), 1))
+    _lib.check(ctx.lib.ocmps_ground_state_dmrg(ctx.h, L, D, int(Npart), float(J), float(U), min(int(maxBondDim), cap), float(threshold),
+                                               int(nsweeps), out.h, C.byref(e), _pd(sweeps)))
+    return (out, e.value, sweeps) if return_info else out
+
+
 def overlapC(a: DeviceMPS, b: DeviceMPS) -> complex:
     """<a|b>, first argument conjugated (ITensor ``overlapC``)."""
     out = np.zeros(2)

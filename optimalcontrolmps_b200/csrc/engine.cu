@@ -1722,6 +1722,21 @@ int ocmps_store_correlations(ocmps_store* store, int slot, const double* op_tabl
   return lease.finish();
 }
 
+// The start state of both ground-state generators, the reference's product state |0..0 1..1> (include/InitializeState.hpp:24-38):
+// one boson on each of the last Npart sites.
+static int upload_product_state(ocmps_mps* out, int L, int D, int Npart) {
+  std::vector<int> dims(L + 1, 1), q(L + 1, 0);
+  std::vector<double> t((size_t)2 * L * D, 0.0);
+  int tot = 0;
+  for (int j = 0; j < L; ++j) {
+    const int occ = j >= L - Npart ? 1 : 0;
+    t[((size_t)j * D + occ) * 2] = 1.0;
+    tot += occ;
+    q[j + 1] = tot;
+  }
+  return ocmps_mps_upload(out, dims.data(), q.data(), t.data(), 0, 2);
+}
+
 // Bose-Hubbard ground state on the device engine (the role of include/InitializeState.hpp:18-117 in the reference:
 // psi_init / psi_target of every main program and test come from it).  The reference runs ITensor's DMRG; here the SAME
 // Trotter-step kernels that do the real-time evolution run in imaginary time: gates exp(-tau h), on-site factors
@@ -1742,21 +1757,10 @@ int ocmps_ground_state(ocmps_ctx* ctx, int L, int D, int Npart, double J, double
   if (cutoff < 0.0) cutoff = 1e-9;
   CK(cudaSetDevice(ctx->dev));
   const int cap = out->lay.cap;
-  {   // product state |0..0 1..1>
-    std::vector<int> dims(L + 1, 1), q(L + 1, 0);
-    std::vector<double> t((size_t)2 * L * D, 0.0);
-    int tot = 0;
-    for (int j = 0; j < L; ++j) {
-      const int occ = j >= L - Npart ? 1 : 0;
-      t[((size_t)j * D + occ) * 2] = 1.0;
-      tot += occ;
-      q[j + 1] = tot;
-    }
-    int rc = ocmps_mps_upload(out, dims.data(), q.data(), t.data(), 0, 2);
-    if (rc) return rc;
-  }
+  int rc = upload_product_state(out, L, D, Npart);
+  if (rc) return rc;
   ocmps_store* tmp = nullptr;
-  int rc = ocmps_store_create(ctx, L, D, cap, 1, &tmp);
+  rc = ocmps_store_create(ctx, L, D, cap, 1, &tmp);
   if (rc) return rc;
   // operator table: 0 = Adag, 1 = A; entries (i, Adag, i+1, A)
   std::vector<double> ops((size_t)2 * D * D, 0.0);
@@ -1820,6 +1824,177 @@ int ocmps_ground_state(ocmps_ctx* ctx, int L, int D, int Npart, double J, double
   if (rc) return rc;
   if (energy_out) *energy_out = e_prev;
   if (steps_out) *steps_out = total_steps;
+  return OCMPS_OK;
+}
+
+// Bose-Hubbard ground state by two-site DMRG on the device (the reference's InitializeState, include/InitializeState.hpp:18-117,
+// runs ITensor's DMRG).  The algorithm is the oracle's ground_state_dmrg: the product start state of ocmps_ground_state, the
+// bond-dimension-4 MPO of the chain, right environments first, then left->right and right->left half sweeps over the bonds.  At
+// each bond: a Lanczos solve of H_eff theta (4 Krylov vectors, full reorthogonalisation, charge-allowed entries only), the gate
+// decomposition with ITensor's truncation (cutoff, maxm of the sweep), the environment update.  Bond dimensions follow the
+// reference's schedule 10, 20, 50, maxm.  There is no noise term (the reference adds none to its energy either; the oracle has
+// none).  One sweep is enqueued without host synchronisation; the host reads the last Ritz value of every sweep.
+int ocmps_ground_state_dmrg(ocmps_ctx* ctx, int L, int D, int Npart, double J, double U, int maxm, double cutoff, int nsweeps,
+                            ocmps_mps* out, double* energy_out, double* sweep_energies) {
+  if (!ctx || !out) return fail(OCMPS_ERR_INVALID, "null argument");
+  if (L < 2 || Npart < 0 || Npart > L) return fail(OCMPS_ERR_INVALID, "ground_state_dmrg: needs L >= 2 and 0 <= Npart <= L (the reference supports one boson per site at most in its initial guess)");
+  if (out->lay.L != L || out->lay.D != D) return fail(OCMPS_ERR_INVALID, "ground_state_dmrg: output MPS has another shape");
+  if (nsweeps < 1) return fail(OCMPS_ERR_INVALID, "ground_state_dmrg: nsweeps must be >= 1");
+  if (maxm < 1) maxm = out->lay.cap;
+  if (maxm > out->lay.cap) return fail(OCMPS_ERR_CAPACITY, "ground_state_dmrg: maxm exceeds the capacity of the output MPS");
+  if (cutoff < 0.0) cutoff = 1e-9;
+  CK(cudaSetDevice(ctx->dev));
+  int rc = upload_product_state(out, L, D, Npart);
+  if (rc) return rc;
+  ocmps_mps* m = out;
+  const Layout& lay = m->lay;
+  const int cap = lay.cap;
+  WsLease lease;
+  rc = lease.acquire(ctx, L, D, cap, 1);
+  if (rc) return rc;
+  Workspace* ws = lease[0];
+  cudaStream_t s = ws->stream;
+
+  // buffers of this call: environments (3 channels per bond and side), Krylov vectors V_0..V_3 + W, the Ritz vector X,
+  // boundary products Y / Z of H_eff, products T / T' of the environment update
+  long long vmax = 1, tmax = 1;
+  for (int b = 0; b + 2 <= L; ++b) vmax = std::max(vmax, (long long)lay.capb[b] * D * D * lay.capb[b + 2]);
+  for (int j = 0; j < L; ++j) tmax = std::max(tmax, (long long)lay.capb[j] * D * lay.capb[j + 1]);
+  const long long estride = (long long)cap * cap;
+  struct Bufs {
+    cplx *EL = nullptr, *ER = nullptr, *V = nullptr, *X = nullptr, *Y = nullptr, *Z = nullptr, *T = nullptr, *T2 = nullptr;
+    GemmDesc* descs = nullptr;
+    KrylovState* ks = nullptr;
+    double *partial = nullptr, *energies = nullptr;
+    cudaStream_t s = nullptr;
+    ~Bufs() {
+      if (s) cudaStreamSynchronize(s);
+      cudaFree(EL); cudaFree(ER); cudaFree(V); cudaFree(X); cudaFree(Y); cudaFree(Z); cudaFree(T); cudaFree(T2);
+      cudaFree(descs); cudaFree(ks); cudaFree(partial); cudaFree(energies);
+    }
+  } B;
+  B.s = s;
+  const size_t env_bytes = sizeof(cplx) * (size_t)(L + 1) * 3 * estride;
+  CK(cudaMalloc(&B.EL, env_bytes));
+  CK(cudaMalloc(&B.ER, env_bytes));
+  CK(cudaMalloc(&B.V, sizeof(cplx) * (size_t)(DMRG_KRYLOV + 1) * vmax));
+  CK(cudaMalloc(&B.X, sizeof(cplx) * (size_t)vmax));
+  CK(cudaMalloc(&B.Y, sizeof(cplx) * (size_t)3 * vmax));
+  CK(cudaMalloc(&B.Z, sizeof(cplx) * (size_t)3 * vmax));
+  CK(cudaMalloc(&B.T, sizeof(cplx) * (size_t)3 * tmax));
+  CK(cudaMalloc(&B.T2, sizeof(cplx) * (size_t)3 * tmax));
+  CK(cudaMalloc(&B.descs, sizeof(GemmDesc) * 13));
+  CK(cudaMalloc(&B.ks, sizeof(KrylovState)));
+  CK(cudaMalloc(&B.partial, sizeof(double) * 2 * 128 * (DMRG_KRYLOV + 1)));
+  CK(cudaMalloc(&B.energies, sizeof(double) * (nsweeps + 1)));
+  // the boundary environments (left of site 0, right of site L-1) are 1 x 1 and hold no term: zero
+  CK(cudaMemsetAsync(B.EL, 0, env_bytes, s));
+  CK(cudaMemsetAsync(B.ER, 0, env_bytes, s));
+  CK(cudaMemsetAsync(B.ks, 0, sizeof(KrylovState), s));
+  cplx* W = B.V + (size_t)DMRG_KRYLOV * vmax;
+  GemmDesc* hdescs = B.descs;          // [0, 6) H_eff, [6, 12) environment update, [12] two-site merge
+  GemmDesc* edescs = B.descs + 6;
+  GemmDesc* mdesc = B.descs + 12;
+  auto env = [&](cplx* E, int b) { return E + (size_t)b * 3 * estride; };
+
+  // ER[j] (sites >= j) from ER[j+1] and the right isometry at site j; EL[j+1] (sites <= j) from EL[j] and the left isometry at j
+  auto grow_right = [&](int j) {
+    launch_env_update(edescs, 1, m->site(j), env(B.ER, j + 1), env(B.ER, j), B.T, B.T2, tmax, estride, m->dim(j), m->dim(j + 1), D,
+                      J, U, lay.capb[j], lay.capb[j + 1], s);
+    g_ocmps_launches += 4;
+  };
+  auto grow_left = [&](int j) {
+    launch_env_update(edescs, 0, m->site(j), env(B.EL, j), env(B.EL, j + 1), B.T, B.T2, tmax, estride, m->dim(j), m->dim(j + 1), D,
+                      J, U, lay.capb[j], lay.capb[j + 1], s);
+    g_ocmps_launches += 4;
+  };
+  // theta of sites b, b+1 -> X, normalised -> V_0 (new Krylov space)
+  auto merge_start = [&](int b) {
+    const int* dl = m->dim(b);
+    const int* dr = m->dim(b + 2);
+    const int nmax = lay.capb[b] * D * D * lay.capb[b + 2];
+    launch_merge_setup(mdesc, m->site(b), m->site(b + 1), B.X, dl, m->dim(b + 1), dr, D, s);
+    launch_zgemm(mdesc, 1, lay.capb[b] * D, D * lay.capb[b + 2], s);
+    launch_krylov_dot(B.X, 0, 1, B.X, dl, dr, D, nullptr, B.partial, s);
+    launch_krylov_init(B.X, B.V, dl, dr, D, B.ks, B.partial, nmax, s);
+    g_ocmps_launches += 4;
+  };
+  auto heff = [&](int b, const cplx* Vin) {
+    launch_heff(hdescs, Vin, W, B.Y, B.Z, vmax, env(B.EL, b), env(B.ER, b + 2), estride, m->dim(b), m->dim(b + 2), m->q(b), m->q(b + 2),
+                D, J, U, B.ks, lay.capb[b], lay.capb[b + 2], s);
+    g_ocmps_launches += 4;
+  };
+  // Lanczos solve at bond b (sites b, b+1), gate decomposition, the theta of the next bond left in the MPS
+  auto bond_step = [&](int b, bool left, int mm) {
+    const int* dl = m->dim(b);
+    const int* dr = m->dim(b + 2);
+    const int nmax = lay.capb[b] * D * D * lay.capb[b + 2];
+    merge_start(b);
+    for (int it = 0; it < DMRG_KRYLOV; ++it) {
+      const cplx* Vit = B.V + (size_t)it * vmax;
+      heff(b, Vit);
+      launch_krylov_dot(Vit, 0, 1, W, dl, dr, D, B.ks, B.partial, s);
+      launch_krylov_alpha(B.V, vmax, it, W, dl, dr, D, B.ks, B.partial, nmax, s);
+      g_ocmps_launches += 2;
+      if (it == DMRG_KRYLOV - 1) break;            // the last residual is not needed
+      launch_krylov_dot(B.V, vmax, it + 1, W, dl, dr, D, B.ks, B.partial, s);
+      launch_krylov_reorth(B.V, vmax, it + 1, W, dl, dr, D, B.ks, B.partial, nmax, s);
+      launch_krylov_dot(W, 0, 1, W, dl, dr, D, B.ks, B.partial, s);
+      launch_krylov_next(B.V, vmax, it, W, dl, dr, D, B.ks, B.partial, nmax, s);
+      g_ocmps_launches += 4;
+    }
+    launch_krylov_ritz(B.ks, s);
+    launch_krylov_combine(B.V, vmax, B.X, dl, dr, D, B.ks, nmax, s);
+    launch_krylov_dot(B.X, 0, 1, B.X, dl, dr, D, nullptr, B.partial, s);
+    launch_krylov_scale(B.X, dl, dr, D, B.partial, nmax, s);
+    g_ocmps_launches += 4;
+    const int j1 = b, j2 = b + 1, bm = b + 1;
+    DecompArgs a;
+    a.kind = left ? DK_GATE_LEFT : DK_GATE_RIGHT;
+    a.D = D;
+    a.dimL = dl; a.dimR = dr; a.qL = m->q(b); a.qR = m->q(b + 2);
+    a.dimNew = m->dim(bm); a.qNew = m->q(bm);
+    a.X = B.X;
+    a.iso = left ? m->other(j1) : m->other(j2);
+    a.partner = left ? m->other(j2) : m->other(j1);
+    a.nb_in = nullptr; a.nb_out = nullptr; a.dimNb = nullptr; a.qNb = nullptr;
+    const TruncParams tp{cutoff, mm, 1, 0, lay.capb[bm], 1};
+    const int capV = left ? lay.capb[b + 2] : lay.capb[b];
+    const int capC = left ? lay.capb[b] : lay.capb[b + 2];
+    run_decomp(ws, a, tp, capV, capC, lay.capb[bm], s);
+    m->cur[j1] ^= 1; m->cur[j2] ^= 1;
+  };
+
+  for (int j = L - 1; j >= 2; --j) grow_right(j);
+  const int sched[4] = {10, 20, 50, maxm};
+  std::vector<double> h_e(nsweeps + 1, 0.0);
+  for (int sw = 0; sw < nsweeps && !rc; ++sw) {
+    const int mm = std::min(maxm, sched[std::min(sw, 3)]);
+    for (int b = 0; b <= L - 2; ++b) {
+      bond_step(b, true, mm);
+      if (b < L - 2) grow_left(b);
+    }
+    for (int b = L - 2; b >= 0; --b) {
+      bond_step(b, false, mm);
+      if (b > 0) grow_right(b + 1);
+    }
+    CK(cudaMemcpyAsync(B.energies + sw, &B.ks->ritz, sizeof(double), cudaMemcpyDeviceToDevice, s));
+    CK(cudaMemcpyAsync(&h_e[sw], B.energies + sw, sizeof(double), cudaMemcpyDeviceToHost, s));
+    rc = lease.finish();               // waits for the sweep; reports (and clears) what its kernels flagged
+  }
+  if (rc) return rc;
+  // <psi|H|psi> of the returned state: one H_eff application on the final two-site tensor (bond 0, after truncation)
+  merge_start(0);
+  heff(0, B.V);
+  launch_krylov_dot(B.V, 0, 1, W, m->dim(0), m->dim(2), D, B.ks, B.partial, s);
+  launch_partial_total(B.partial, B.energies + nsweeps, s);
+  g_ocmps_launches += 2;
+  CK(cudaMemcpyAsync(&h_e[nsweeps], B.energies + nsweeps, sizeof(double), cudaMemcpyDeviceToHost, s));
+  rc = lease.finish();
+  if (rc) return rc;
+  m->llim = 0; m->rlim = 2;
+  if (energy_out) *energy_out = h_e[nsweeps];
+  if (sweep_energies) for (int sw = 0; sw < nsweeps; ++sw) sweep_energies[sw] = h_e[sw];
   return OCMPS_OK;
 }
 

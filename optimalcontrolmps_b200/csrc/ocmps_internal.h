@@ -173,6 +173,43 @@ void launch_overlap_site_op(cplx* T, long long t_stride, const GemmDesc* descs, 
                             int max_elems, cudaStream_t s);
 void launch_overlap_final(const cplx* E, long long e_stride, int batch, int withK, cplx* out, cudaStream_t s);
 
+// ---- two-site DMRG (dmrg.cu) ----
+constexpr int DMRG_KRYLOV = 4;      // Lanczos vectors per bond
+struct KrylovState {                // device-resident state of the Lanczos solve of one bond
+  double alpha[DMRG_KRYLOV], beta[DMRG_KRYLOV];
+  double y[DMRG_KRYLOV];            // Ritz vector in the Krylov basis
+  double ritz;                      // lowest Ritz value
+  int nk;                           // Krylov vectors in use
+  int stop;                         // breakdown: the remaining Krylov launches of this bond do nothing
+};
+// W = H_eff V on the two-site tensor of bonds dimL / dimR: environments EL (left bond) and ER (right bond), three channels at
+// stride estride each; Y, Z: scratch of 3 x ystride elements each; descs: 6 GemmDesc
+void launch_heff(GemmDesc* descs, const cplx* V, cplx* W, cplx* Y, cplx* Z, long long ystride, const cplx* EL, const cplx* ER,
+                 long long estride, const int* dimL, const int* dimR, const int* qL, const int* qR, int D, double J, double U,
+                 const KrylovState* ks, int capL, int capR, cudaStream_t s);
+// environment of bond j+1 from bond j (side 0, A = left isometry of site j) or of bond j from bond j+1 (side 1, A = right
+// isometry of site j); dimL / dimR are bonds j, j+1; T, T2: scratch of 3 x tstride elements each; descs: 6 GemmDesc
+void launch_env_update(GemmDesc* descs, int side, const cplx* A, const cplx* Ein, cplx* Eout, cplx* T, cplx* T2, long long tstride,
+                       long long estride, const int* dimL, const int* dimR, int D, double J, double U, int capL, int capR,
+                       cudaStream_t s);
+// Lanczos steps on two-site vectors of bonds dimL / dimR; partial: (DMRG_KRYLOV + 1) x 128 x 2 doubles; ks = nullptr in
+// krylov_dot: run even after a breakdown
+void launch_krylov_dot(const cplx* V, long long vstride, int nvec, const cplx* w, const int* dimL, const int* dimR, int D,
+                       const KrylovState* ks, double* partial, cudaStream_t s);
+void launch_krylov_init(const cplx* X, cplx* V0, const int* dimL, const int* dimR, int D, KrylovState* ks, const double* partial,
+                        int max_elems, cudaStream_t s);
+void launch_krylov_alpha(const cplx* V, long long vstride, int it, cplx* w, const int* dimL, const int* dimR, int D, KrylovState* ks,
+                         const double* partial, int max_elems, cudaStream_t s);
+void launch_krylov_reorth(const cplx* V, long long vstride, int nvec, cplx* w, const int* dimL, const int* dimR, int D,
+                          const KrylovState* ks, const double* partial, int max_elems, cudaStream_t s);
+void launch_krylov_next(cplx* V, long long vstride, int it, const cplx* w, const int* dimL, const int* dimR, int D, KrylovState* ks,
+                        const double* partial, int max_elems, cudaStream_t s);
+void launch_krylov_ritz(KrylovState* ks, cudaStream_t s);
+void launch_krylov_combine(const cplx* V, long long vstride, cplx* X, const int* dimL, const int* dimR, int D, const KrylovState* ks,
+                           int max_elems, cudaStream_t s);
+void launch_krylov_scale(cplx* X, const int* dimL, const int* dimR, int D, const double* partial, int max_elems, cudaStream_t s);
+void launch_partial_total(const double* partial, double* out, cudaStream_t s);   // real part of the first dot product
+
 // K|psi>: builds the bond-dimension-2chi tensors
 void launch_applyK_expand(const cplx* A, cplx* B, const int* dimL_in, const int* dimR_in, const int* qL_in, const int* qR_in,
                           int* dimL_out, int* dimR_out, int* qL_out, int* qR_out, int D, int site, int L, int max_elems,
