@@ -23,6 +23,7 @@ class BH_tDMRG {
   IQMPO propagatorDeriv(const double& control_n) const;
   double getTstep() const;
   Args getArgs() const;
+  double getJ() const { return J_; }
   // GPU-side accessors used by OptimalControl
   ocmps_stepper* handle() const { return p_ ? p_->h : nullptr; }
   int capacity() const { return cap_; }

@@ -40,6 +40,7 @@ class OptimalControl {
   stdvec calcAnalyticGradient(const stdvec& control, const bool new_control = true);
   rowmat calcHessian(const stdvec& control, const bool new_control = true);
   stdvec calcFidelityForAllT(const stdvec& control, const bool new_control = true);
+  void calcEnergyForAllT(const stdvec& control, const bool new_control, bool variance, stdvec& E, stdvec& var);
 
  public:
   // psi_t / xi_t / xiHlist live in device stores owned by this object; a copy would have to duplicate gigabytes of
@@ -69,6 +70,10 @@ class OptimalControl {
   stdvec getAnalyticGradient(const stdvec& control, const bool new_control = true);
   rowmat getHessian(const stdvec& control, const bool new_control = true);
   stdvec getFidelityForAllT(const stdvec& control, const bool new_control = true);
+  // <psi_i|H(u_i)|psi_i> / <psi_i|psi_i> on the psi slices (the excess energy along the ramp) and its variance <H^2> - <H>^2;
+  // J from the stepper, caching as getFidelityForAllT (new_control = false keeps the slices, the control only sets u_i)
+  stdvec getEnergyForAllT(const stdvec& control, const bool new_control = true);
+  stdvec getEnergyVarianceForAllT(const stdvec& control, const bool new_control = true);
   rowmat getControlJacobian() const;
 };
 #endif

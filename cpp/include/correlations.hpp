@@ -173,4 +173,33 @@ inline std::vector<double> entanglementEntropy(itensor::SiteSet const& sites, it
   return S;
 }
 
+// Energy <psi|H|psi> / <psi|psi> of H = -J sum (a_i adag_{i+1} + h.c.) + U/2 sum n_i(n_i-1) (include/InitializeState.hpp:41-50) and
+// its variance <H^2> - <H>^2 (zero on an eigenstate), by the transfer-matrix chain of the MPO on the device.  Any gauge.
+namespace ocmps_detail {
+inline void energy_moments(itensor::IQMPS& psi, double J, double U, const double* shift, int second_moment, double* m) {
+  using namespace itensor;
+  ocmps_store* store = nullptr;
+  ocmps_check(ocmps_store_create(default_context(), psi.N(), psi.D(), psi.capacity(), 1, &store), "ocmps_store_create");
+  int rc = ocmps_store_put(store, 0, psi.handle());
+  if (!rc) rc = ocmps_store_energy_moments(store, 0, 1, J, &U, shift, second_moment, m);
+  ocmps_store_destroy(store);
+  ocmps_check(rc, "ocmps_store_energy_moments");
+}
+}  // namespace ocmps_detail
+
+inline double energy(itensor::SiteSet const& sites, itensor::IQMPS& psi, double J, double U) {
+  (void)sites;
+  double m[3] = {0.0, 0.0, 0.0};
+  ocmps_detail::energy_moments(psi, J, U, nullptr, 0, m);
+  return m[1] / m[0];
+}
+
+inline double energyVariance(itensor::SiteSet const& sites, itensor::IQMPS& psi, double J, double U) {
+  const double E = energy(sites, psi, J, U);
+  double m[3] = {0.0, 0.0, 0.0};
+  ocmps_detail::energy_moments(psi, J, U, &E, 1, m);
+  const double h1 = m[1] / m[0];
+  return m[2] / m[0] - h1 * h1;
+}
+
 #endif

@@ -199,6 +199,22 @@ template <class TS> stdvec OptimalControl<TS>::calcFidelityForAllT(const stdvec&
   return f;
 }
 
+template <class TS>
+void OptimalControl<TS>::calcEnergyForAllT(const stdvec& u, const bool new_control, bool variance, stdvec& E, stdvec& var) {
+  if (new_control) { calculatedXi = false; calcPsi(u); }
+  std::vector<double> m(3 * N, 0.0);
+  ocmps_check(ocmps_store_energy_moments(psi_t->h, 0, (int)N, timeStepper.getJ(), u.data(), nullptr, 0, m.data()), "ocmps_store_energy_moments");
+  E.assign(N, 0.0);
+  for (size_t i = 0; i < N; ++i) E[i] = m[3 * i + 1] / m[3 * i];
+  if (!variance) return;
+  ocmps_check(ocmps_store_energy_moments(psi_t->h, 0, (int)N, timeStepper.getJ(), u.data(), E.data(), 1, m.data()), "ocmps_store_energy_moments");
+  var.assign(N, 0.0);
+  for (size_t i = 0; i < N; ++i) {
+    const double h1 = m[3 * i + 1] / m[3 * i];
+    var[i] = m[3 * i + 2] / m[3 * i] - h1 * h1;
+  }
+}
+
 // ---- public API (:495-589) ----
 template <class TS> void OptimalControl<TS>::propagatePsi(const stdvec& c) { calcPsi(GRAPE ? c : basis.convertControl(c)); }
 template <class TS> double OptimalControl<TS>::getCost(const stdvec& c, const bool nc) {
@@ -214,6 +230,16 @@ template <class TS> rowmat OptimalControl<TS>::getHessian(const stdvec& c, const
 }
 template <class TS> stdvec OptimalControl<TS>::getFidelityForAllT(const stdvec& c, const bool nc) {
   return GRAPE ? calcFidelityForAllT(c, nc) : calcFidelityForAllT(basis.convertControl(c, nc), nc);
+}
+template <class TS> stdvec OptimalControl<TS>::getEnergyForAllT(const stdvec& c, const bool nc) {
+  stdvec E, var;
+  calcEnergyForAllT(GRAPE ? c : basis.convertControl(c, nc), nc, false, E, var);
+  return E;
+}
+template <class TS> stdvec OptimalControl<TS>::getEnergyVarianceForAllT(const stdvec& c, const bool nc) {
+  stdvec E, var;
+  calcEnergyForAllT(GRAPE ? c : basis.convertControl(c, nc), nc, true, E, var);
+  return var;
 }
 template <class TS> rowmat OptimalControl<TS>::getControlJacobian() const {
   if (!GRAPE) return basis.getControlJacobian();

@@ -153,6 +153,14 @@ int ocmps_store_correlations(ocmps_store* store, int slot, const double* op_tabl
  * S = -sum_{p > 1e-12} p ln p over the density-matrix eigenvalues): out[z*(L-1) + (i-1)] for bond i = 1..L-1 of the slices
  * first..first+count-1.  Works on a copy (the store is not modified); slices must have their centre at site 1. */
 int ocmps_store_entanglement_entropy(ocmps_store* store, int first, int count, double* out /* count*(L-1) */);
+/* Energy moments of the slices first..first+count-1 under H(U_z) - c_z, H(U) = -J sum (a_i adag_{i+1} + h.c.) + U/2 sum n_i(n_i-1)
+ * (the Hamiltonian of include/InitializeState.hpp:41-50 and of the stepper at control value U):
+ * out[3z+0] = <psi|psi>,  out[3z+1] = <psi|H-c|psi>,  out[3z+2] = <psi|(H-c)^2|psi>  (raw, not divided by the norm).
+ * U: count values (the control value of each slice); shift: count values or NULL (c = 0).
+ * second_moment = 0 runs the 4-channel chain of the MPO and leaves out[3z+2] untouched; 1 runs the 16-channel chain of its
+ * square (about 4x the work).  Any gauge.  A slice's results do not depend on the other slices of the call. */
+int ocmps_store_energy_moments(ocmps_store* store, int first, int count, double J, const double* U, const double* shift,
+                               int second_moment, double* out /* 3*count */);
 /* xiHlist[i] = exactApplyMPO(K, xi_t[i], args) for all i (:300-303) */
 int ocmps_store_apply_K(ocmps_stepper* st, ocmps_store* in, int Nt, ocmps_store* out);
 /* calcHessianRow (:252-279) for `nrows` rows listed in `rows`: for every row r the raw ingredients are returned,

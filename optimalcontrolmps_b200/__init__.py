@@ -13,8 +13,8 @@ import os as _os
 _os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")
 
 from .api import (Args, BH_tDMRG, InitializeState, InitializeStateDMRG, BoseHubbard, Context, ControlBasis, ControlBasisFactory, DeviceMPS, IQMPS,
-                  OptimalControl, SeedGenerator, SliceStore, batch_cost_gradient, overlapC, overlapC_K, site_operator)
+                  OptimalControl, SeedGenerator, SliceStore, batch_cost_gradient, energy, overlapC, overlapC_K, site_operator)
 from ._lib import OcmpsError, LIB_PATH
 
 __all__ = ["Args", "BH_tDMRG", "InitializeState", "InitializeStateDMRG", "BoseHubbard", "Context", "ControlBasis", "ControlBasisFactory", "DeviceMPS", "IQMPS",
-           "OptimalControl", "SeedGenerator", "batch_cost_gradient", "SliceStore", "overlapC", "overlapC_K", "site_operator", "OcmpsError", "LIB_PATH"]
+           "OptimalControl", "SeedGenerator", "batch_cost_gradient", "energy", "SliceStore", "overlapC", "overlapC_K", "site_operator", "OcmpsError", "LIB_PATH"]

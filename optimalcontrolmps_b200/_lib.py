@@ -23,6 +23,7 @@ SYMBOLS = [
     "ocmps_forward_sweep", "ocmps_backward_sweep", "ocmps_sweep_pair", "ocmps_sweep_batch", "ocmps_backward_sweep_divT",
     "ocmps_store_overlaps", "ocmps_store_divT", "ocmps_store_apply_K", "ocmps_hessian_rows", "ocmps_hessian_eval",
     "ocmps_store_site_expectations", "ocmps_store_entanglement_entropy", "ocmps_store_correlations",
+    "ocmps_store_energy_moments",
 ]
 
 
@@ -93,6 +94,7 @@ def load():
         "ocmps_store_site_expectations": (i, [vp, i, i, pd, i, pd, pd]),
         "ocmps_store_entanglement_entropy": (i, [vp, i, i, pd]),
         "ocmps_store_correlations": (i, [vp, i, pd, i, pi, i, pd]),
+        "ocmps_store_energy_moments": (i, [vp, i, i, d, pd, pd, i, pd]),
         "ocmps_ground_state": (i, [vp, i, i, i, d, d, i, d, d, vp, pd, pi]),
         "ocmps_ground_state_dmrg": (i, [vp, i, i, i, d, d, i, d, i, vp, pd, pd]),
     }

@@ -269,6 +269,39 @@ class SliceStore:
         _lib.check(self.ctx.lib.ocmps_store_site_expectations(self.h, first, count, _pd(diags), len(opnames), _pd(out), _pd(nrm)))
         return (out, nrm) if return_norm else out
 
+    # ---- energy of the Bose-Hubbard Hamiltonian H(U) = -J sum (a_i adag_{i+1} + h.c.) + U/2 sum n_i(n_i-1) ----
+    def energyMoments(self, J: float, U, first=0, count=None, shift=None, second_moment=True):
+        """Raw moments of H(U_z) - c_z on the slices first..first+count-1 in one transfer-matrix pass over the MPO channels:
+        arrays ``(norm2, h1, h2)`` of <psi|psi>, <psi|H-c|psi> and <psi|(H-c)^2|psi> (nothing divided by the norm; h2 is NaN
+        with ``second_moment=False``, which runs the 4-channel chain at about a quarter of the cost).  ``U`` and ``shift`` are
+        scalars or one value per slice.  Any gauge."""
+        count = self.nslots - first if count is None else count
+        u = np.ascontiguousarray(np.broadcast_to(np.asarray(U, dtype=np.float64), (count,)))
+        c = None if shift is None else np.ascontiguousarray(np.broadcast_to(np.asarray(shift, dtype=np.float64), (count,)))
+        out = np.full((count, 3), np.nan)
+        _lib.check(self.ctx.lib.ocmps_store_energy_moments(self.h, int(first), int(count), float(J), _pd(u),
+                                                            None if c is None else _pd(c), 1 if second_moment else 0, _pd(out)))
+        return out[:, 0].copy(), out[:, 1].copy(), out[:, 2].copy()
+
+    def energies(self, J: float, U, first=0, count=None, variance=False):
+        """<psi|H(U_z)|psi> / <psi|psi> of every slice; with ``variance=True`` ``(E, var)``, var = <H^2> - <H>^2 from a second pass
+        of the 16-channel chain shifted by E (so that no E^2 cancels against <H^2>)."""
+        n, h1, _ = self.energyMoments(J, U, first, count, second_moment=False)
+        E = h1 / n
+        if not variance:
+            return E
+        n2, g1, g2 = self.energyMoments(J, U, first, count, shift=E, second_moment=True)
+        return E, g2 / n2 - (g1 / n2) ** 2
+
+
+def energy(psi: "DeviceMPS", J: float, U: float, variance: bool = False):
+    """<psi|H(U)|psi> / <psi|psi> of a device MPS (``(E, var)`` with ``variance=True``), e.g. the convergence check of a DMRG ground
+    state: the variance <H^2> - <H>^2 vanishes on an eigenstate."""
+    store = SliceStore(psi.ctx, psi.L, psi.D, psi.chi_cap, 1)
+    store.put(0, psi)
+    out = store.energies(J, [U], 0, 1, variance=variance)
+    return (float(out[0][0]), float(out[1][0])) if variance else float(out[0])
+
 
 def site_operator(opname: str, D: int) -> np.ndarray:
     """<t|Op|s> of the site operators of include/BH_sites.h:129-171 as a real D x D matrix ("Id" is the true identity, which
@@ -410,6 +443,9 @@ class BH_tDMRG:
 
     def getArgs(self) -> Args:
         return self.args
+
+    def getJ(self) -> float:
+        return self.J
 
     def propagatorDeriv(self, control_n: float = 0.0):
         """The constant MPO K = sum_j 1/2 n_j(n_j-1) (src/BH_tDMRG.cpp:10-14,238-241); it lives inside the
@@ -859,6 +895,24 @@ class OptimalControl:
         if self.GRAPE:
             return self._calcFidelityForAllT(control, new_control)
         return self._calcFidelityForAllT(self.basis.convertControl(control, new_control), new_control)
+
+    # <psi_i|H(u_i)|psi_i> / <psi_i|psi_i> along the ramp: the excess energy over the instantaneous ground state, and its variance.
+    # Same caching as getFidelityForAllT: new_control=True re-propagates psi; with False the cached slices are kept and the
+    # control passed only sets u_i.
+    def _calcEnergyForAllT(self, control, new_control=True, variance=False):
+        u = self._u(control)
+        if new_control:
+            self.calculatedXi = False
+            self._calcPsi(u)
+        return self.psi_t.energies(self.timeStepper.getJ(), u, 0, self.N, variance=variance)
+
+    def getEnergyForAllT(self, control, new_control: bool = True) -> stdvec:
+        u = control if self.GRAPE else self.basis.convertControl(control, new_control)
+        return [float(e) for e in self._calcEnergyForAllT(u, new_control)]
+
+    def getEnergyVarianceForAllT(self, control, new_control: bool = True) -> stdvec:
+        u = control if self.GRAPE else self.basis.convertControl(control, new_control)
+        return [float(v) for v in self._calcEnergyForAllT(u, new_control, variance=True)[1]]
 
     def getControlJacobian(self):
         if self.GRAPE:

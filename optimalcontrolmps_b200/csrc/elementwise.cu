@@ -324,21 +324,22 @@ __device__ __forceinline__ const int* side_dims(const OvlSide& s, int z) {
   return s.dims + (long long)(s.use_ptrs ? 0 : (s.slot0 + z)) * s.dims_stride;
 }
 
-// Per batch entry z and site j: T = E . B_j   (nE*chiA x D*chiB')   and  E'_c = A_j^H . T_c  for c < nE.
+// Per batch entry z and site j: T = E . B_j   (nE*chiA x D*chiB')   and  E'_c = A_j^H . Tm_c  for c < nE, with nE environment
+// channels stacked along M.  Tm is T itself, or a second buffer (same stride) that a channel-mixing kernel fills from T.
 // descs layout: [0*batch + z] the T gemm, [(1+c)*batch + z] the E' gemms.
-__global__ void overlap_plan_kernel(GemmDesc* descs, OvlSide bra, OvlSide ket, int site, int batch, int D, int withK, cplx* E_in,
-                                    cplx* E_out, cplx* T, long long e_stride, long long t_stride) {
+__global__ void overlap_plan_kernel(GemmDesc* descs, OvlSide bra, OvlSide ket, int site, int batch, int D, int nE, cplx* E_in,
+                                    cplx* E_out, cplx* T, const cplx* Tm, long long e_stride, long long t_stride) {
   const int z = blockIdx.x * blockDim.x + threadIdx.x;
   if (z >= batch) return;
   const int* da = side_dims(bra, z);
   const int* db = side_dims(ket, z);
   const int aL = da[site], aR = da[site + 1], bL = db[site], bR = db[site + 1];
-  const int nE = withK ? 2 : 1;
   const cplx* A = side_site(bra, z, site);
   const cplx* B = side_site(ket, z, site);
   cplx* Ei = E_in + z * e_stride;
   cplx* Eo = E_out + z * e_stride;
   cplx* Tz = T + z * t_stride;
+  const cplx* Tmz = Tm + z * t_stride;
   GemmDesc g;
   g.pad = 0;
   // T (nE*aL x D*bR) = E (nE*aL x bL) . B (bL x D*bR)
@@ -347,9 +348,9 @@ __global__ void overlap_plan_kernel(GemmDesc* descs, OvlSide bra, OvlSide ket, i
   g.C = Tz; g.ldc = D * bR; g.M = nE * aL; g.N = D * bR; g.K = bL;
   descs[z] = g;
   for (int c = 0; c < nE; ++c) {
-    // E'_c (aR x bR) = A^H (aL*D x aR)^H . T_c (aL*D x bR)
+    // E'_c (aR x bR) = A^H (aL*D x aR)^H . Tm_c (aL*D x bR)
     g.A = A; g.opA = 1; g.lda = aR;
-    g.B = Tz + (long long)c * aL * D * bR; g.opB = 0; g.ldb = bR;
+    g.B = Tmz + (long long)c * aL * D * bR; g.opB = 0; g.ldb = bR;
     g.C = Eo + (long long)c * aR * bR; g.ldc = bR; g.M = aR; g.N = bR; g.K = aL * D;
     descs[(1 + c) * batch + z] = g;
   }
@@ -450,6 +451,84 @@ __global__ void overlap_final_kernel(const cplx* E, long long e_stride, int batc
   const int z = blockIdx.x * blockDim.x + threadIdx.x;
   if (z >= batch) return;
   out[z] = E[z * e_stride + (withK ? 1 : 0)];
+}
+
+// ---- energy moments: the transfer-matrix chain of <psi|W..W|psi> (4 channels) or <psi|(W x W)..(W x W)|psi> (16 channels) ----
+// Left boundary: every channel 0 except the start channel nch-1 (MPO state 3, "nothing placed yet"), which is 1.
+__global__ void energy_init_kernel(cplx* E, long long e_stride, int batch, int nch) {
+  const int z = blockIdx.x * blockDim.x + threadIdx.x;
+  if (z >= batch) return;
+  for (int c = 0; c < nch; ++c) E[z * e_stride + c] = make_double2(c == nch - 1 ? 1.0 : 0.0, 0.0);
+}
+
+__device__ __forceinline__ double energy_factor(const EnergyTable& tab, int f, int t, int s, int D, double U, double cL) {
+  switch (f) {
+    case ENERGY_F_ID: return t == s ? 1.0 : 0.0;
+    case ENERGY_F_A: return tab.A[t * D + s];
+    case ENERGY_F_ADAG: return tab.Adag[t * D + s];
+    default: return t == s ? 0.5 * U * t * (t - 1) - cL : 0.0;   // ENERGY_F_ONSITE
+  }
+}
+
+// T'_v[l][t][r] = sum_{k: dst_k = v} sum_s O_k[t][s] T_{src_k}[l][s][r] for every target channel v, with the transition operators
+// O_k = coef_k F1_k F2_k built per slice (its U_z, c_z / L) in shared memory.  T and T' are [c][l][s][r] with channel stride
+// aL*D*bR.  One thread per (l, r) column; the table is sorted by target channel, so a target is accumulated in registers and
+// written once, in a fixed order.
+template <int D>
+__global__ void __launch_bounds__(256) energy_mix_kernel(const cplx* __restrict__ T, cplx* __restrict__ Tm, long long t_stride,
+                                                         const GemmDesc* __restrict__ descs, const double* __restrict__ uc,
+                                                         const EnergyTable tab) {
+  __shared__ double sO[ENERGY_MAX_TRANS * D * D];
+  const int z = blockIdx.y;
+  const double U = uc[2 * z], cL = uc[2 * z + 1];
+  for (int i = threadIdx.x; i < tab.nt * D * D; i += blockDim.x) {
+    const int k = i / (D * D), t = (i / D) % D, s = i % D;
+    double acc = 0.0;
+    for (int m = 0; m < D; ++m) acc += energy_factor(tab, tab.f1[k], t, m, D, U, cL) * energy_factor(tab, tab.f2[k], m, s, D, U, cL);
+    sO[i] = tab.coef[k] * acc;
+  }
+  __syncthreads();
+  const int nch = tab.nch;
+  const GemmDesc g = descs[z];
+  const int aL = g.M / nch, N = g.N, bR = N / D;
+  const long long cs = (long long)aL * N;
+  const cplx* __restrict__ Tz = T + z * t_stride;
+  cplx* __restrict__ Tmz = Tm + z * t_stride;
+  const long long total = (long long)aL * bR;
+  for (long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
+    const long long off = (e / bR) * N + (e % bR);
+    int k = 0;
+    for (int v = 0; v < nch; ++v) {
+      double ar[D], ai[D];
+#pragma unroll
+      for (int t = 0; t < D; ++t) { ar[t] = 0.0; ai[t] = 0.0; }
+      for (; k < tab.nt && tab.dst[k] == v; ++k) {
+        const cplx* col = Tz + tab.src[k] * cs + off;
+        cplx x[D];
+#pragma unroll
+        for (int s = 0; s < D; ++s) x[s] = col[(long long)s * bR];
+        const double* O = sO + k * D * D;
+#pragma unroll
+        for (int t = 0; t < D; ++t)
+#pragma unroll
+          for (int s = 0; s < D; ++s) { const double o = O[t * D + s]; ar[t] += o * x[s].x; ai[t] += o * x[s].y; }
+      }
+      cplx* out = Tmz + v * cs + off;
+#pragma unroll
+      for (int t = 0; t < D; ++t) out[(long long)t * bR] = make_double2(ar[t], ai[t]);
+    }
+  }
+}
+
+// Right boundary (1 x 1 per channel): out[3z] = <psi|psi>, out[3z+1] = <psi|H-c|psi>, out[3z+2] = <psi|(H-c)^2|psi> (16 channels;
+// 0 with 4).  Channel (a, b) of the 16 is 4a+b; the end state is 0, so (3,3) carries the norm, (0,3) one factor of H-c, (0,0) two.
+__global__ void energy_final_kernel(const cplx* E, long long e_stride, int batch, int nch, double* out) {
+  const int z = blockIdx.x * blockDim.x + threadIdx.x;
+  if (z >= batch) return;
+  const cplx* Ez = E + z * e_stride;
+  out[3 * z + 0] = Ez[nch - 1].x;
+  out[3 * z + 1] = Ez[nch == 16 ? 3 : 0].x;
+  out[3 * z + 2] = nch == 16 ? Ez[0].x : 0.0;
 }
 
 // ---- K|psi>: B[(l,a), s, (r,b)] = A[l,s,r] W[a,b,s], W = [[1,0],[k_s,1]], boundaries pick row 1 / column 0 ----
@@ -578,7 +657,33 @@ void launch_unpack_copy(const cplx* src_base, SitePtrs dst, SiteOffs offs, const
 
 void launch_overlap_plan(GemmDesc* descs, const OvlSide& bra, const OvlSide& ket, int site, int batch, int D, int withK,
                          cplx* E_in, cplx* E_out, cplx* T, long long e_stride, long long t_stride, cudaStream_t s) {
-  overlap_plan_kernel<<<(batch + 63) / 64, 64, 0, s>>>(descs, bra, ket, site, batch, D, withK, E_in, E_out, T, e_stride, t_stride);
+  overlap_plan_kernel<<<(batch + 63) / 64, 64, 0, s>>>(descs, bra, ket, site, batch, D, withK ? 2 : 1, E_in, E_out, T, T, e_stride,
+                                                       t_stride);
+}
+void launch_overlap_plan_channels(GemmDesc* descs, const OvlSide& bra, const OvlSide& ket, int site, int batch, int D, int nch,
+                                  cplx* E_in, cplx* E_out, cplx* T, const cplx* Tmix, long long e_stride, long long t_stride,
+                                  cudaStream_t s) {
+  overlap_plan_kernel<<<(batch + 63) / 64, 64, 0, s>>>(descs, bra, ket, site, batch, D, nch, E_in, E_out, T, Tmix, e_stride, t_stride);
+}
+void launch_energy_init(cplx* E, long long e_stride, int batch, int nch, cudaStream_t s) {
+  energy_init_kernel<<<(batch + 63) / 64, 64, 0, s>>>(E, e_stride, batch, nch);
+}
+void launch_energy_mix(const cplx* T, cplx* Tmix, long long t_stride, const GemmDesc* descs, int batch, int D, const double* uc,
+                       const EnergyTable& tab, int max_cols, cudaStream_t s) {
+  const dim3 grid(grid_for(max_cols, 256, 128), batch);
+  switch (D) {
+    case 1: energy_mix_kernel<1><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 2: energy_mix_kernel<2><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 3: energy_mix_kernel<3><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 4: energy_mix_kernel<4><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 5: energy_mix_kernel<5><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 6: energy_mix_kernel<6><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    case 7: energy_mix_kernel<7><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+    default: energy_mix_kernel<8><<<grid, 256, 0, s>>>(T, Tmix, t_stride, descs, uc, tab); break;
+  }
+}
+void launch_energy_final(const cplx* E, long long e_stride, int batch, int nch, double* out, cudaStream_t s) {
+  energy_final_kernel<<<(batch + 63) / 64, 64, 0, s>>>(E, e_stride, batch, nch, out);
 }
 void launch_overlap_local_expect(const GemmDesc* descs, const OvlSide& bra, int site, int batch, int D, const double* ops, int nops,
                                  double* out, int L, cudaStream_t s) {

@@ -161,6 +161,19 @@ struct Workspace {
   cplx* d_out = nullptr;       // overlap results (device)
   int obatch = 0;
   long long e_stride = 0, t_stride = 0;
+  // energy moments: nch-channel environments, T and the channel-mixed T' (kept apart from the overlap buffers, so that a
+  // 16-channel pass does not grow what every overlap call of the workspace carries)
+  struct EnergyBufs {
+    cplx* E[2] = {nullptr, nullptr};
+    cplx* T = nullptr;
+    cplx* Tm = nullptr;
+    GemmDesc* descs = nullptr;
+    double* uc = nullptr;        // (U_z, c_z / L) per batch entry
+    double* out = nullptr;       // 3 per batch entry
+    long long e_elems = 0, t_elems = 0, ndescs = 0;   // allocated sizes (elements of each E / of T and of T')
+    int batch = 0;
+    long long e_stride = 0, t_stride = 0;             // of the current call
+  } en;
   // work states
   ocmps_mps* work = nullptr;
   ocmps_mps* big = nullptr;    // 2*cap bonds, for K|psi>
@@ -301,6 +314,27 @@ int ensure_overlap_bufs(Workspace* w, int batch, int capA, int capB) {
   return OCMPS_OK;
 }
 
+// Energy-moment buffers for `batch` entries of nch channels at capacity cap (the workspace's stream is idle).  Sized in
+// elements, so that the 4- and 16-channel passes, whose batches are cut to the same byte budget, share one allocation.
+int ensure_energy_bufs(Workspace* w, int batch, int nch, int cap) {
+  auto& b = w->en;
+  const long long es = (long long)nch * cap * cap, ts = (long long)nch * cap * w->D * cap;
+  b.e_stride = es; b.t_stride = ts;
+  if (b.e_elems >= es * batch && b.t_elems >= ts * batch && b.ndescs >= (1LL + nch) * batch && b.batch >= batch) return OCMPS_OK;
+  cudaFree(b.E[0]); cudaFree(b.E[1]); cudaFree(b.T); cudaFree(b.Tm); cudaFree(b.descs); cudaFree(b.uc); cudaFree(b.out);
+  b.E[0] = b.E[1] = b.T = b.Tm = nullptr; b.descs = nullptr; b.uc = b.out = nullptr;
+  b.e_elems = std::max(b.e_elems, es * batch); b.t_elems = std::max(b.t_elems, ts * batch);
+  b.ndescs = std::max(b.ndescs, (1LL + nch) * batch); b.batch = std::max(b.batch, batch);
+  CK(cudaMalloc(&b.E[0], sizeof(cplx) * b.e_elems));
+  CK(cudaMalloc(&b.E[1], sizeof(cplx) * b.e_elems));
+  CK(cudaMalloc(&b.T, sizeof(cplx) * b.t_elems));
+  CK(cudaMalloc(&b.Tm, sizeof(cplx) * b.t_elems));
+  CK(cudaMalloc(&b.descs, sizeof(GemmDesc) * b.ndescs));
+  CK(cudaMalloc(&b.uc, sizeof(double) * 2 * b.batch));
+  CK(cudaMalloc(&b.out, sizeof(double) * 3 * b.batch));
+  return OCMPS_OK;
+}
+
 void free_ws(Workspace* w) {
   if (!w) return;
   cudaFree(w->theta); cudaFree(w->cbuf); cudaFree(w->db.dw); cudaFree(w->db.vec_idx); cudaFree(w->db.comp_idx);
@@ -322,6 +356,8 @@ void free_ws(Workspace* w) {
   free_mps(w->tmpK);
   if (w->rowstore) { cudaFree(w->rowstore->data); cudaFree(w->rowstore->dims); cudaFree(w->rowstore->q); delete w->rowstore; }
   cudaFree(w->E[0]); cudaFree(w->E[1]); cudaFree(w->T); cudaFree(w->odescs); cudaFree(w->d_out);
+  cudaFree(w->en.E[0]); cudaFree(w->en.E[1]); cudaFree(w->en.T); cudaFree(w->en.Tm); cudaFree(w->en.descs); cudaFree(w->en.uc);
+  cudaFree(w->en.out);
   cudaFree(w->d_status); cudaFree(w->d_div);
   if (w->work) w->work->ctx = nullptr;      // (owned by the workspace, whose graphs are gone with it: no bookkeeping)
   if (w->big) w->big->ctx = nullptr;
@@ -1718,6 +1754,109 @@ int ocmps_store_correlations(ocmps_store* store, int slot, const double* op_tabl
   }
   cudaStreamSynchronize(s);
   cudaFree(d_ops); cudaFree(d_sel);
+  if (rc) return rc;
+  return lease.finish();
+}
+
+// Energy moments of resident slices under H(U_z) - c_z, the Hamiltonian of include/InitializeState.hpp:41-50 (and of the
+// stepper at control value U): one transfer-matrix pass over all L sites per slice with the environments of the MPO channels
+// (4 for W, 16 for W x W, see EnergyTable), batched over the slices.  Per site: T = E . B_j for all channels in one gemm per
+// slice, the channel mixing on the physical index, then E'_v = A_j^H . T'_v.  No gauge is assumed; nothing is divided by the
+// norm.  Slices are batched in chunks whose T and T' fit ENERGY_CHUNK_BYTES; every slice's reductions run in a fixed order
+// that does not depend on the chunk, so a slice gives the same bits alone or in any batch.
+constexpr long long ENERGY_CHUNK_BYTES = 1LL << 30;
+constexpr int ENERGY_MAX_BATCH = 256;
+
+static EnergyTable energy_table(int D, double J, int second_moment) {
+  struct Entry { int a, b, f; double coef; };
+  const Entry W[7] = {{0, 0, ENERGY_F_ID, 1.0},    {3, 3, ENERGY_F_ID, 1.0},  {3, 0, ENERGY_F_ONSITE, 1.0}, {3, 1, ENERGY_F_A, -J},
+                      {3, 2, ENERGY_F_ADAG, -J},   {1, 0, ENERGY_F_ADAG, 1.0}, {2, 0, ENERGY_F_A, 1.0}};
+  EnergyTable t;
+  memset(&t, 0, sizeof(t));
+  t.nch = second_moment ? 16 : 4;
+  for (int s = 1; s < D; ++s) {
+    t.A[(s - 1) * D + s] = std::sqrt((double)s);      // a|s> = sqrt(s) |s-1>
+    t.Adag[s * D + (s - 1)] = std::sqrt((double)s);   // adag|s-1> = sqrt(s) |s>
+  }
+  std::vector<Entry> tr;                              // (src, dst, f1, coef) and f2 below
+  std::vector<int> f2;
+  for (int i = 0; i < 7; ++i) {
+    if (!second_moment) { tr.push_back(W[i]); f2.push_back(ENERGY_F_ID); continue; }
+    for (int k = 0; k < 7; ++k) {
+      tr.push_back({4 * W[i].a + W[k].a, 4 * W[i].b + W[k].b, W[i].f, W[i].coef * W[k].coef});
+      f2.push_back(W[k].f);
+    }
+  }
+  std::vector<int> order(tr.size());
+  for (size_t i = 0; i < order.size(); ++i) order[i] = (int)i;
+  std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return tr[x].b < tr[y].b; });
+  t.nt = (int)tr.size();
+  for (int k = 0; k < t.nt; ++k) {
+    const Entry& e = tr[order[k]];
+    t.src[k] = e.a; t.dst[k] = e.b; t.f1[k] = e.f; t.f2[k] = f2[order[k]]; t.coef[k] = e.coef;
+  }
+  return t;
+}
+
+int ocmps_store_energy_moments(ocmps_store* store, int first, int count, double J, const double* U, const double* shift,
+                               int second_moment, double* out) {
+  if (!store || !U || !out || count < 1 || first < 0 || first > store->nslots - count || (second_moment != 0 && second_moment != 1))
+    return fail(OCMPS_ERR_INVALID, "bad argument");
+  if (!std::isfinite(J)) return fail(OCMPS_ERR_INVALID, "energy_moments: J is not finite");
+  for (int z = 0; z < count; ++z)
+    if (!std::isfinite(U[z]) || (shift && !std::isfinite(shift[z])))
+      return fail(OCMPS_ERR_INVALID, "energy_moments: U or shift is not finite");
+  ocmps_ctx* ctx = store->ctx;
+  const Layout& lay = store->lay;
+  const int L = lay.L, D = lay.D;
+  const EnergyTable tab = energy_table(D, J, second_moment);
+  const int nch = tab.nch;
+  CK(cudaSetDevice(ctx->dev));
+  WsLease lease;
+  int rc = lease.acquire(ctx, L, D, lay.cap, 1);
+  if (rc) return rc;
+  Workspace* ws = lease[0];
+  cudaStream_t s = ws->stream;
+  const long long slice_bytes = 2LL * nch * lay.cap * D * lay.cap * (long long)sizeof(cplx);   // T and T'
+  const int chunk = (int)std::max(1LL, std::min<long long>({(long long)ENERGY_MAX_BATCH, (long long)count, ENERGY_CHUNK_BYTES / slice_bytes}));
+  CK(cudaStreamSynchronize(s));
+  rc = ensure_energy_bufs(ws, chunk, nch, lay.cap);
+  if (rc) return rc;
+  const auto& b = ws->en;
+  std::vector<double> h_uc(2 * (size_t)chunk), h_out(3 * (size_t)chunk);
+  for (int z0 = 0; z0 < count && !rc; z0 += chunk) {
+    const int nb = std::min(chunk, count - z0);
+    for (int z = 0; z < nb; ++z) {
+      h_uc[2 * z] = U[z0 + z];
+      h_uc[2 * z + 1] = shift ? shift[z0 + z] / L : 0.0;
+    }
+    if (cudaMemcpyAsync(b.uc, h_uc.data(), sizeof(double) * 2 * nb, cudaMemcpyHostToDevice, s) != cudaSuccess) {
+      rc = fail(OCMPS_ERR_CUDA, "energy_moments: copy failed"); break;
+    }
+    const OvlSide side = side_of_store(store, first + z0);
+    launch_energy_init(b.E[0], b.e_stride, nb, nch, s);
+    int cur = 0;
+    for (int j = 0; j < L; ++j) {
+      launch_overlap_plan_channels(b.descs, side, side, j, nb, D, nch, b.E[cur], b.E[1 - cur], b.T, b.Tm, b.e_stride, b.t_stride, s);
+      launch_zgemm(b.descs, nb, nch * lay.capb[j], D * lay.capb[j + 1], s);
+      launch_energy_mix(b.T, b.Tm, b.t_stride, b.descs, nb, D, b.uc, tab, lay.capb[j] * lay.capb[j + 1], s);
+      launch_zgemm(b.descs + nb, nch * nb, lay.capb[j + 1], lay.capb[j + 1], s);
+      cur = 1 - cur;
+      g_ocmps_launches += 4;
+    }
+    launch_energy_final(b.E[cur], b.e_stride, nb, nch, b.out, s);
+    g_ocmps_launches += 2;
+    if (cudaMemcpyAsync(h_out.data(), b.out, sizeof(double) * 3 * nb, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+        cudaStreamSynchronize(s) != cudaSuccess) {
+      rc = fail(OCMPS_ERR_CUDA, "energy_moments: copy failed"); break;
+    }
+    for (int z = 0; z < nb; ++z) {
+      out[3 * (z0 + z) + 0] = h_out[3 * z + 0];
+      out[3 * (z0 + z) + 1] = h_out[3 * z + 1];
+      if (second_moment) out[3 * (z0 + z) + 2] = h_out[3 * z + 2];
+    }
+  }
+  cudaStreamSynchronize(s);
   if (rc) return rc;
   return lease.finish();
 }

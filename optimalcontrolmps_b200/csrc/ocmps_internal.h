@@ -172,6 +172,29 @@ void launch_overlap_kfix(cplx* T, long long t_stride, const GemmDesc* descs, int
 void launch_overlap_site_op(cplx* T, long long t_stride, const GemmDesc* descs, int batch, int D, const double* op_table, const int* sel,
                             int max_elems, cudaStream_t s);
 void launch_overlap_final(const cplx* E, long long e_stride, int batch, int withK, cplx* out, cudaStream_t s);
+// nch environment channels; the E' gemms read Tmix (pass T for no channel mixing).  launch_overlap_plan is nch = withK ? 2 : 1.
+void launch_overlap_plan_channels(GemmDesc* descs, const OvlSide& bra, const OvlSide& ket, int site, int batch, int D, int nch,
+                                  cplx* E_in, cplx* E_out, cplx* T, const cplx* Tmix, long long e_stride, long long t_stride,
+                                  cudaStream_t s);
+
+// Energy moments of H(U) - c with the bond-dimension-4 MPO W of the Bose-Hubbard chain (MPO states 3 = nothing placed, 1 / 2 =
+// a / adag placed, 0 = done): W[0,0] = W[3,3] = I, W[3,0] = U/2 N(N-1) - c/L, W[3,1] = -J A, W[3,2] = -J Adag, W[1,0] = Adag,
+// W[2,0] = A.  A transition src -> dst of the channel chain applies coef * F1 F2 (F2 = I for the 4 channels of W; the 16
+// channels (a,b) of W x W apply W[a,a'] W[b,b']).
+enum { ENERGY_F_ID = 0, ENERGY_F_A = 1, ENERGY_F_ADAG = 2, ENERGY_F_ONSITE = 3 };
+constexpr int ENERGY_MAX_TRANS = 49;
+struct EnergyTable {
+  int nch, nt;                                   // channels (4 or 16), transitions (7 or 49), sorted by dst
+  int src[ENERGY_MAX_TRANS], dst[ENERGY_MAX_TRANS];
+  int f1[ENERGY_MAX_TRANS], f2[ENERGY_MAX_TRANS];
+  double coef[ENERGY_MAX_TRANS];
+  double A[OCMPS_MAX_D * OCMPS_MAX_D], Adag[OCMPS_MAX_D * OCMPS_MAX_D];   // <t|a|s>, <t|adag|s>, row-major D x D
+};
+void launch_energy_init(cplx* E, long long e_stride, int batch, int nch, cudaStream_t s);
+// uc: per batch entry (U_z, c_z / L); max_cols: capacity bound of aL * bR
+void launch_energy_mix(const cplx* T, cplx* Tmix, long long t_stride, const GemmDesc* descs, int batch, int D, const double* uc,
+                       const EnergyTable& tab, int max_cols, cudaStream_t s);
+void launch_energy_final(const cplx* E, long long e_stride, int batch, int nch, double* out, cudaStream_t s);
 
 // ---- two-site DMRG (dmrg.cu) ----
 constexpr int DMRG_KRYLOV = 4;      // Lanczos vectors per bond
